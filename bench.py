@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the hot path's headline measurement (see DESIGN.md "Measurement").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1], the QuantizeLinear up_proj operands):
     x  bf16 [8192, 4096]   A8 per-token   SymQuantizer forward + STE backward
@@ -102,6 +102,30 @@ def make_inputs(seed: int):
     gx = torch.randn(T_TOK, K_IN, generator=g)
     gw = torch.randn(N_OUT, K_IN, generator=g)
     return [t.bfloat16() for t in (x, w, gx, gw)]
+
+
+DUMP_ROWS = 512   # rows of each operand that --dump-outputs writes: 4 files of 512 x 4096 float32 = 32 MB
+
+
+def dump_rows():
+    """The fixed, seeded row indices of x and of W that --dump-outputs writes (sorted)."""
+    g = torch.Generator().manual_seed(0)
+    return (torch.randperm(T_TOK, generator=g)[:DUMP_ROWS].sort().values,
+            torch.randperm(N_OUT, generator=g)[:DUMP_ROWS].sort().values)
+
+
+def dump_outputs(out_dir: str, y_x, y_w, grad_x, grad_w):
+    """--dump-outputs: what one step hands its caller (fake-quantized x and W, the STE gradients of both) as
+    float32 DIR/<name>.npy.  Whole rows, the unit each scale is computed over, at the dump_rows() sample
+    (the same rows for an output and its gradient), so that two builds or the two arms can be compared
+    element for element."""
+    import numpy as np
+
+    rows_x, rows_w = dump_rows()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t, rows in (("y_x", y_x, rows_x), ("y_w", y_w, rows_w), ("grad_x", grad_x, rows_x),
+                          ("grad_w", grad_w, rows_w)):
+        np.save(os.path.join(out_dir, name + ".npy"), t.index_select(0, rows.to(t.device)).float().cpu().numpy())
 
 
 # ----------------------------------------------------------------------------
@@ -601,6 +625,8 @@ def run_b200(args):
         ms_total = float(t.item())
     ms_step = ms_total / K
     value = world * STEP_BYTES / (ms_step * 1e-3) / 1e9
+    if args.dump_outputs and rank == 0:   # the buffers hold what the last timed step wrote
+        dump_outputs(args.dump_outputs, step.yx, step.yw, step.dx, step.dw)
 
     # ---- region 2: per-kernel durations for the roofline.  An event record between
     # two kernels costs ~4 us of serialisation, so each kernel is timed as K
@@ -807,17 +833,20 @@ def run_b200(args):
 # ----------------------------------------------------------------------------
 # CPU port of the reference (cpu_baseline leg and --impl reference arm)
 # ----------------------------------------------------------------------------
-def run_cpu_port(hx, hw, hgx, hgw, budget_s: float, steps: int | None = None, warmup: int = 1):
+def run_cpu_port(hx, hw, hgx, hgw, budget_s: float, steps: int | None = None, warmup: int = 1, last=None):
     """Times oracle/torch_chain.py (the torch-eager port of utils_quant.py) on
-    the host cores over the SAME workload; a step = fwd+bwd of x and of W."""
+    the host cores over the SAME workload; a step = fwd+bwd of x and of W.
+    A dict passed as `last` receives the last step's (y, grad) of "x" and "w"."""
     from oracle import torch_chain as tc
 
     cores = os.cpu_count() or 1
     torch.set_num_threads(cores)
 
     def step():
-        tc.fwd_bwd(hx, hgx, A_BITS, True, CLIP)
-        tc.fwd_bwd(hw, hgw, W_BITS, True, CLIP)
+        ox = tc.fwd_bwd(hx, hgx, A_BITS, True, CLIP)
+        ow = tc.fwd_bwd(hw, hgw, W_BITS, True, CLIP)
+        if last is not None:
+            last["x"], last["w"] = ox, ow
 
     for _ in range(warmup):
         step()
@@ -847,7 +876,10 @@ def run_reference(args):
     world = int(os.environ.get("WORLD_SIZE", str(args.gpus)))
     hx, hw, hgx, hgw = make_inputs(1234)
     K, W = args.steps, max(args.warmup, 3)      # the same K / W the b200 arm reports (~0.1-0.3 s per step)
-    cb = run_cpu_port(hx, hw, hgx, hgw, budget_s=0.0, steps=K, warmup=W)
+    last = {} if args.dump_outputs else None
+    cb = run_cpu_port(hx, hw, hgx, hgw, budget_s=0.0, steps=K, warmup=W, last=last)
+    if last is not None:
+        dump_outputs(args.dump_outputs, last["x"][0], last["w"][0], last["x"][1], last["w"][1])
     line = {
         "impl": "reference", "metric": METRIC, "value": cb["value"], "unit": "GB/s",
         "n_gpus": world, "steps": K, "warmup": W,
@@ -883,7 +915,12 @@ def main():
                     help="model of the QAT-step extra: 7b = BASELINE configs[3], 13b = configs[4] (W4A8KV8)")
     ap.add_argument("--hang-dump-s", type=int, default=int(os.environ.get("BENCH_HANG_DUMP_S", "600")),
                     help="dump every thread's stack and exit if the run is still going after this many seconds")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (a fixed sample of "
+                         f"{DUMP_ROWS} rows per operand) as float32 DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     import faulthandler
 
     # a stuck collective must not sit there until the driver's limit: report where each rank is and exit

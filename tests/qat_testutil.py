@@ -4,11 +4,18 @@ from __future__ import annotations
 import os
 
 import numpy as np
+import pytest
 import torch
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 DTYPES = {"fp32": torch.float32, "bf16": torch.bfloat16}
 _cache = {}
+
+# A checkout of the original LLM-QAT project (the directory holding its models/ package).  The tests that import
+# its code run only where QAT_B200_REFERENCE names one; what it computed on the stored cases is in golden/.
+REFERENCE = os.path.abspath(os.environ["QAT_B200_REFERENCE"]) if os.environ.get("QAT_B200_REFERENCE") else ""
+needs_reference = pytest.mark.skipif(not (REFERENCE and os.path.isdir(os.path.join(REFERENCE, "models"))),
+                                     reason="needs the original project's source: set QAT_B200_REFERENCE to a checkout")
 
 
 def golden(dtype: str):

@@ -1,9 +1,11 @@
 """The configs 3-5 harness (harness/llama_qat.py) and the oracle-side quant
 module (oracle/ref_module.py).
 
-CPU, build container only (skipped where /root/reference is absent): both are
-pinned to the LIVE reference — ref_module bit for bit against
-models/utils_quant.py, the harness layer against the real LlamaDecoderLayer.
+CPU: both are pinned to the reference's stored outputs (tests/golden/) — ref_module
+bit for bit against what models/utils_quant.py computed, the harness layer in bf16
+against what the real LlamaDecoderLayer computed (layer_bf16.npz).  With a checkout
+of the original project (QAT_B200_REFERENCE) also against its live code, which adds
+the fp32 layer comparison and the model-file binding checks.
 GPU: the harness on llm_qat_b200 vs the harness on the oracle module."""
 import os
 import sys
@@ -12,12 +14,14 @@ import numpy as np
 import pytest
 import torch
 
+import qat_testutil as U
 from harness import llama_qat as H
 from oracle import grid_module as G
 from oracle import ref_module as R
 
-REF = "/root/reference"
-needs_reference = pytest.mark.skipif(not os.path.isdir(REF), reason="live reference only exists in the build container")
+REF = U.REFERENCE
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+needs_reference = U.needs_reference
 
 
 def _ref_modules():
@@ -61,6 +65,52 @@ def test_ref_module_matches_live_reference(dtype):
         oa.backward(go)
         ob.backward(go)
         assert torch.equal(oa, ob) and torch.equal(a.grad, b.grad) and torch.equal(la.weight.grad, lb.weight.grad), kw
+
+
+@pytest.mark.parametrize("dtype", ["fp32", "bf16"])
+def test_ref_module_reproduces_the_reference_goldens(dtype):
+    """ref_module (the eager comparator of the GPU tests and of bench.py) against what the original
+    models/utils_quant.py computed on the CPU (tests/golden/quant_*.npz, oracle/gen_golden.py), bit for bit:
+    both quantizers' forward on every stored case, their STE backward for every stored clip, and
+    QuantizeLinear's output, input gradient and weight gradient for every stored bit-width combination,
+    the W1 / W2 weight path included."""
+    g = U.golden(dtype)
+    tdt = U.DTYPES[dtype]
+    t = lambda k: U.bits_to_tensor(g[k], dtype)  # noqa: E731
+    quant = {"sym": R.SymQuantizer, "asym": R.AsymQuantizer}
+    n = 0
+    for q, key, bits, lw in U.quant_cases(g):
+        y = quant[q].apply(t(f"in/{key}"), torch.tensor([-2.0, 2.0]), bits, lw)
+        k = f"y/{q}/{key}/b{bits}/{'lw' if lw else 'row'}"
+        assert U.mismatches(U.tensor_bits(y), g[k], dtype) == 0, k
+        n += 1
+    for q, key, lw, lo, hi, k in U.clip_cases(g):
+        x = t(f"in/{key}").requires_grad_(True)      # bit widths as oracle/gen_golden.py ran the backward
+        quant[q].apply(x, torch.tensor([lo, hi]), 2 if q == "sym" else 3, lw).backward(t(f"grad/{key}"))
+        assert U.mismatches(U.tensor_bits(x.grad), g[k], dtype) == 0, k
+        n += 1
+    for tag in [k.split("/")[-1] for k in g.files if k.startswith("lin/out/")]:
+        body = tag.replace("_wlw", "")
+        w_bits, rest = int(body[1:body.index("a")]), body[body.index("a") + 1:]
+        lin = R.QuantizeLinear(192, 80, symmetric=rest[-1] == "s", w_bits=w_bits, a_bits=int(rest[:-1]),
+                               weight_layerwise=tag.endswith("_wlw")).to(tdt)
+        with torch.no_grad():
+            lin.weight.copy_(t("lin/w"))
+        x = t("lin/x").requires_grad_(True)
+        out = lin(x)
+        out.backward(t("lin/g"))
+        for what, v in (("out", out), ("gx", x.grad), ("gw", lin.weight.grad)):
+            assert U.mismatches(U.tensor_bits(v), g[f"lin/{what}/{tag}"], dtype) == 0, (what, tag)
+            n += 1
+    for k in [k for k in g.files if k.startswith("lowbit/weff/")]:
+        tag = k.split("/")[-1]
+        lin = R.QuantizeLinear(192, 40, w_bits=int(tag[1]), a_bits=32, weight_layerwise=tag.endswith("_lw")).to(tdt)
+        with torch.no_grad():
+            lin.weight.copy_(t("lowbit/w"))
+        w_eff = lin(torch.eye(192, dtype=tdt)).detach().t().contiguous()   # as oracle/gen_golden.py recovers it
+        assert U.mismatches(U.tensor_bits(w_eff), g[k], dtype) == 0, k
+        n += 1
+    assert n == 178, n
 
 
 @needs_reference
@@ -240,7 +290,7 @@ def test_reference_model_file_builds_on_the_product_module():
     code = r'''
 import sys
 sys.dont_write_bytecode = True
-sys.path.insert(0, "/root/reference"); sys.path.insert(0, %r)
+sys.path.insert(0, %r); sys.path.insert(0, %r)
 import llm_qat_b200
 import models                                   # the reference package
 llm_qat_b200.install()                          # models.utils_quant -> the product
@@ -258,7 +308,7 @@ assert att.act_quantizer_k is llm_qat_b200.SymQuantizer and att.kv_bits == 4
 keys = sorted(model.state_dict().keys())
 assert all(not k.endswith("_qat_wfeed") for k in keys) and "model.layers.0.mlp.up_proj.weight" in keys
 print("ok", len(keys))
-''' % os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+''' % (REF, ROOT)
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)
     assert r.returncode == 0 and r.stdout.startswith("ok"), r.stdout + r.stderr[-3000:]
 
@@ -314,7 +364,7 @@ def test_fuse_model_binds_the_unmodified_reference_model():
     code = r'''
 import sys
 sys.dont_write_bytecode = True
-sys.path.insert(0, "/root/reference"); sys.path.insert(0, %r)
+sys.path.insert(0, %r); sys.path.insert(0, %r)
 import torch
 import llm_qat_b200
 import models
@@ -361,7 +411,7 @@ llm_qat_b200.unfuse_model(model)
 assert "forward" not in lay.self_attn.__dict__ and "forward" not in model.model.__dict__
 assert lay.self_attn.forward.__func__ is cls_fwd
 print("ok")
-''' % os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+''' % (REF, ROOT)
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)
     assert r.returncode == 0 and r.stdout.startswith("ok"), r.stdout + r.stderr[-3000:]
 
@@ -574,7 +624,7 @@ def test_fuse_model_glue_on_the_real_model_file_with_emulated_kernels():
     code = r'''
 import sys, math
 sys.dont_write_bytecode = True
-sys.path.insert(0, "/root/reference"); sys.path.insert(0, %r)
+sys.path.insert(0, %r); sys.path.insert(0, %r)
 import torch
 import models
 from oracle import ref_module as R
@@ -649,6 +699,6 @@ llm_qat_b200.unfuse_model(model)
 l3, _, _ = run()
 assert torch.equal(l3, l0)
 print("ok")
-''' % os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+''' % (REF, ROOT)
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=900)
     assert r.returncode == 0 and r.stdout.strip().endswith("ok"), r.stdout[-2000:] + r.stderr[-4000:]

@@ -136,21 +136,24 @@ def test_bf16_reciprocal_quotient_proof(tmp_path):
         assert r.returncode == 0 and " 0 mismatches" in r.stdout, r.stdout + r.stderr
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="live reference only exists in the build container")
-def test_oracle_fuzz_matches_live_reference():
-    """The oracle against the UNMODIFIED reference (imported read-only) on the seeded fuzz cases
-    the GPU parity test uses: forward values and STE gradients, bit for bit."""
+def _live_reference():
+    """The original's models/utils_quant.py, imported read-only from the QAT_B200_REFERENCE checkout."""
+    import importlib
     import sys
 
+    sys.dont_write_bytecode = True
+    if U.REFERENCE not in sys.path:
+        sys.path.insert(0, U.REFERENCE)
+    uq = importlib.import_module("models.utils_quant")
+    assert uq.__file__.startswith(U.REFERENCE)
+    return uq
+
+
+def _fuzz_vs(uq):
+    """The oracle against module `uq`'s SymQuantizer / AsymQuantizer on the seeded fuzz cases the GPU parity
+    test uses: forward values and STE gradients, bit for bit."""
     import torch
 
-    sys.dont_write_bytecode = True
-    if "/root/reference" not in sys.path:
-        sys.path.insert(0, "/root/reference")
-    import importlib
-
-    uq = importlib.import_module("models.utils_quant")
-    assert uq.__file__.startswith("/root/reference")
     clip = torch.tensor([-2.0, 2.0])
     n = 0
     for seed in range(12):
@@ -166,21 +169,12 @@ def test_oracle_fuzz_matches_live_reference():
     assert n == 72
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="live reference only exists in the build container")
-def test_oracle_lowbit_edge_cases_match_live_reference(monkeypatch):
-    """The oracle's W1 / W2 weight path against the UNMODIFIED reference on the edge-row cases the GPU
+def _lowbit_edge_cases_vs(uq, monkeypatch):
+    """The oracle's W1 / W2 weight path against module `uq`'s QuantizeLinear on the edge-row cases the GPU
     test uses; the effective weight is captured where QuantizeLinear.forward hands it to F.linear."""
-    import sys
-
     import torch
     import torch.nn as nn
 
-    sys.dont_write_bytecode = True
-    if "/root/reference" not in sys.path:
-        sys.path.insert(0, "/root/reference")
-    import importlib
-
-    uq = importlib.import_module("models.utils_quant")
     captured = {}
     orig = nn.functional.linear
 
@@ -201,3 +195,32 @@ def test_oracle_lowbit_edge_cases_match_live_reference(monkeypatch):
             (dtype, rows, cols, bits, lw)
         n += 1
     assert n == 72
+
+
+@U.needs_reference
+def test_oracle_fuzz_matches_live_reference():
+    """The oracle against the UNMODIFIED reference (imported read-only) on the seeded fuzz cases."""
+    _fuzz_vs(_live_reference())
+
+
+@U.needs_reference
+def test_oracle_lowbit_edge_cases_match_live_reference(monkeypatch):
+    """The oracle's W1 / W2 weight path against the UNMODIFIED reference on the edge-row cases."""
+    _lowbit_edge_cases_vs(_live_reference(), monkeypatch)
+
+
+def test_oracle_fuzz_matches_ref_module():
+    """The same fuzz cases against oracle/ref_module.py, which issues the reference's ATen op chain and is
+    held bit for bit to the reference's stored outputs (test_harness.py::test_ref_module_reproduces_the_
+    reference_goldens): the bit widths, widths, ranks and non-finite values the stored cases lack are
+    checked on every machine."""
+    from oracle import ref_module
+
+    _fuzz_vs(ref_module)
+
+
+def test_oracle_lowbit_edge_cases_match_ref_module(monkeypatch):
+    """The W1 / W2 edge-row cases (shapes up to 40000 columns, layerwise included) against oracle/ref_module.py."""
+    from oracle import ref_module
+
+    _lowbit_edge_cases_vs(ref_module, monkeypatch)
