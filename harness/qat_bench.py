@@ -47,15 +47,16 @@ def _timed(fn, warmup, steps):
 
 
 def time_layer(quant, cfg: H.QatConfig, seq=2048, bsz=1, warmup=3, steps=10, device="cuda", seed=1234,
-               autocast=False, fused=False):
+               autocast=False, fused=False, linear=True):
     """Config 3: one LlamaDecoderLayer W4A8KV4 bf16, hidden_states [bsz, seq, H], fwd + bwd.
-    ``fused``: llm_qat_b200.fuse_model on the layer (attention / MLP / RMSNorm kernels)."""
+    ``fused``: llm_qat_b200.fuse_model on the layer (attention / MLP / RMSNorm kernels; ``linear``: its
+    operand route for QuantizeLinear configurations off the int8 grid)."""
     torch.manual_seed(0)
     layer = H.DecoderLayer(cfg, quant).bfloat16().to(device)
     if fused:
         import llm_qat_b200
 
-        llm_qat_b200.fuse_model(layer)
+        llm_qat_b200.fuse_model(layer, linear=linear)
     with torch.no_grad():
         for p in layer.parameters():
             if p.dim() == 2:

@@ -43,6 +43,11 @@ extern "C" {
  * scale, x * s, round, s + 1e-6 and the division all in fp32, and the result is an fp32 tensor
  * (measured on the GPU box: tests/gpu_autocast_probe.py).  qat_sym_fwd only: x bf16, y fp32. */
 #define QAT_BF16_AMP 2
+/* The QAT_BF16_AMP chain followed by the cast autocast's F.linear applies to its operand
+ * (utils_quant.py:250): y = bf16(y_fp32), one more round-to-nearest-even.  This is the exact bf16
+ * operand the reference hands its GEMM under autocast, written at 2 B/elem instead of 4 and without a
+ * separate cast pass.  qat_sym_fwd only: x bf16, y bf16 (codes and mask as for QAT_BF16_AMP). */
+#define QAT_BF16_AMP_CAST 3
 
 /* optional integer-code output */
 #define QAT_CODES_NONE 0

@@ -13,7 +13,7 @@ from ctypes import c_char_p, c_float, c_int, c_int64, c_size_t, c_uint64, c_void
 PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(PKG, "lib", "libqat_b200.so")
 
-QAT_F32, QAT_BF16, QAT_BF16_AMP = 0, 1, 2
+QAT_F32, QAT_BF16, QAT_BF16_AMP, QAT_BF16_AMP_CAST = 0, 1, 2, 3
 CODES_NONE, CODES_I8, CODES_I16 = 0, 1, 2
 ERR_UNSUPPORTED = 1002
 

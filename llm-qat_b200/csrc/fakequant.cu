@@ -874,8 +874,8 @@ template <bool SYM>
 int fwd_entry(const void* x, void* y, void* codes, int codes_kind, float* st0, float* st1,
               uint8_t* mask, float lo, float hi, int64_t rows, int64_t cols, int dtype, int bits,
               void* workspace, size_t workspace_bytes, void* stream, int poison_inf = 0) {
-  QAT_CHECK_ARG(dtype == QAT_F32 || dtype == QAT_BF16 || (SYM && dtype == QAT_BF16_AMP),
-                "dtype must be QAT_F32, QAT_BF16 or (Sym only) QAT_BF16_AMP (got %d)", dtype);
+  QAT_CHECK_ARG(dtype == QAT_F32 || dtype == QAT_BF16 || (SYM && (dtype == QAT_BF16_AMP || dtype == QAT_BF16_AMP_CAST)),
+                "dtype must be QAT_F32, QAT_BF16 or (Sym only) QAT_BF16_AMP / QAT_BF16_AMP_CAST (got %d)", dtype);
   QAT_CHECK_ARG(rows >= 0 && cols >= 0, "negative shape [%lld, %lld]", (long long)rows, (long long)cols);
   QAT_CHECK_ARG(SYM ? (bits >= 2 && bits <= 31) : (bits >= 1 && bits <= 31), "unsupported num_bits %d", bits);
   QAT_CHECK_ARG(!(codes != nullptr && codes_kind == QAT_CODES_I16 && bits > (SYM ? 16 : 15)),
@@ -942,6 +942,7 @@ int fwd_entry(const void* x, void* y, void* codes, int codes_kind, float* st0, f
   if (dtype == QAT_F32) return dispatch<QAT_F32, SYM>(p, pl, st);
   if constexpr (SYM) {
     if (dtype == QAT_BF16_AMP) return dispatch<QAT_BF16_AMP, true>(p, pl, st);
+    if (dtype == QAT_BF16_AMP_CAST) return dispatch<QAT_BF16_AMP_CAST, true>(p, pl, st);
   }
   return dispatch<QAT_BF16, SYM>(p, pl, st);
 }
@@ -950,6 +951,8 @@ int fwd_entry(const void* x, void* y, void* codes, int codes_kind, float* st0, f
 
 int sym_fwd_feed(const void* x, void* codes, float* row_e, uint8_t* mask, float clip_lo, float clip_hi,
                  int64_t rows, int64_t cols, int dtype, int bits, void* stream) {
+  // the feed's codes do not depend on the final cast: QAT_BF16_AMP names the autocast chain here
+  QAT_CHECK_ARG(dtype != QAT_BF16_AMP_CAST, "QAT_BF16_AMP_CAST is a qat_sym_fwd output mode");
   return fwd_entry<true>(x, nullptr, codes, QAT_CODES_I8, nullptr, row_e, mask, clip_lo, clip_hi, rows, cols,
                          dtype, bits, nullptr, 0, stream, /*poison_inf=*/1);
 }

@@ -18,6 +18,10 @@ model file, its classes, parameters and state dict are untouched and ``unfuse_mo
   runs the reference's own forward.
 * MLP (:234-235): silu(gate) * up in one kernel that also emits down_proj's activation codes.
 * RMSNorm (:121-129): one kernel that also emits the codes q/k/v (or gate/up) consume.
+* QuantizeLinear off the int8 grid (W4-A16, weight-only QAT with W1/W2, 9..31-bit weights, activation-only):
+  the reference's exact bf16 operands, from one K1 pass each, contracted on this library's tcgen05 GEMM
+  forward and backward (utils_quant._OperandLinearFn).  Marked per instance (``_qat_operand_route``); the
+  int8-grid configurations keep their own path either way.
 * ``fuse_kd_loss(trainer)``: KDTrainer.ce_loss (utils/kd_trainer.py:42-48) -> fused_ops.kd_loss.
 """
 from __future__ import annotations
@@ -28,7 +32,7 @@ import types
 import torch
 
 from . import fused_ops as F
-from .utils_quant import QuantizeLinear, SymQuantizer, _clip_bounds
+from .utils_quant import QuantizeLinear, SymQuantizer, _clip_bounds, operand_route_config
 
 __all__ = ["fuse_model", "unfuse_model", "fuse_kd_loss", "mark_causal_mask"]
 
@@ -178,10 +182,16 @@ def _bind(mod, name, fn):
     setattr(mod, name, types.MethodType(fn, mod))
 
 
-def fuse_model(model, attention: bool = True, mlp: bool = True, rmsnorm: bool = True):
-    """Rebind the forward of every attention / MLP / RMSNorm module of ``model`` (see module docstring).
+def fuse_model(model, attention: bool = True, mlp: bool = True, rmsnorm: bool = True, linear: bool = True):
+    """Rebind the forward of every attention / MLP / RMSNorm module of ``model`` and, with ``linear``, mark the
+    QuantizeLinear modules the operand route serves (see module docstring; ``linear=False`` clears the marks).
     Returns the model.  Idempotent."""
     for mod in model.modules():
+        if isinstance(mod, QuantizeLinear):
+            if linear and operand_route_config(mod):
+                mod._qat_operand_route = True
+            else:
+                mod.__dict__.pop("_qat_operand_route", None)
         has = lambda *names: all(hasattr(mod, n) for n in names)  # noqa: E731
         if attention and has("q_proj", "k_proj", "v_proj", "o_proj", "rotary_emb", "num_heads", "head_dim"):
             _bind(mod, "forward", _attention_forward)
@@ -209,6 +219,7 @@ def fuse_model(model, attention: bool = True, mlp: bool = True, rmsnorm: bool = 
 
 def unfuse_model(model):
     for mod in model.modules():
+        mod.__dict__.pop("_qat_operand_route", None)
         if "_qat_orig_forward" in mod.__dict__:
             del mod.forward                    # the instance attribute; the class's forward shows again
             del mod._qat_orig_forward

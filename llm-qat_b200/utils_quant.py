@@ -51,7 +51,7 @@ import torch.nn as nn
 
 from . import _lib
 from . import sharding as _sharding
-from ._lib import CODES_I8, CODES_I16, CODES_NONE, QAT_BF16, QAT_BF16_AMP, QAT_F32, check
+from ._lib import CODES_I8, CODES_I16, CODES_NONE, QAT_BF16, QAT_BF16_AMP, QAT_BF16_AMP_CAST, QAT_F32, check
 
 __all__ = ["SymQuantizer", "AsymQuantizer", "QuantizeLinear"]
 
@@ -137,18 +137,20 @@ def _reduction_view(input: torch.Tensor, layerwise: bool):
 
 def fake_quant_forward(input: torch.Tensor, num_bits: int, layerwise: bool, symmetric: bool, *,
                        want_y: bool = True, codes_kind: int = CODES_NONE, want_scales: bool = False,
-                       mask_clip=None, amp: bool = False):
+                       mask_clip=None, amp: bool = False, cast: bool = False):
     """One launch of K1/K2 (or the two-phase K5 for long rows).
 
     Returns ``(y, codes, st0, st1, mask)``; entries not requested are ``None``.
     Sym: st0 = s, st1 = e (dequant divisor).  Asym: st0 = alpha + 1e-8, st1 = beta.
+    ``amp`` with ``cast``: y is the autocast chain's fp32 result cast to bf16 (QAT_BF16_AMP_CAST).
     """
     _require_cuda(input, "fake-quant forward")
     dt = _dtype_code(input)
     if amp:
         if not (symmetric and dt == QAT_BF16):
             raise TypeError("the autocast variant exists for SymQuantizer on bfloat16 tensors only")
-        dt = QAT_BF16_AMP
+        dt = QAT_BF16_AMP_CAST if cast else QAT_BF16_AMP
+    y_fp32 = amp and not cast
     rows, cols = _reduction_view(input, layerwise)
     if input.numel() == 0:
         # what the reference's torch.max does: an empty reduction set raises (IndexError for
@@ -159,13 +161,13 @@ def fake_quant_forward(input: torch.Tensor, num_bits: int, layerwise: bool, symm
                                "Specify the reduction dim with the 'dim' argument.")
         if cols == 0:
             raise IndexError("max(): Expected reduction dim to have non-zero size.")
-        empty = torch.empty(input.shape, dtype=torch.float32 if amp else input.dtype, device=input.device)
+        empty = torch.empty(input.shape, dtype=torch.float32 if y_fp32 else input.dtype, device=input.device)
         return (empty if want_y else None), None, None, None, None
     x = input.detach()
     if not x.is_contiguous():
         x = x.contiguous()
     dev = x.device
-    y = (torch.empty(x.shape, dtype=torch.float32, device=dev) if amp else torch.empty_like(x)) if want_y else None
+    y = (torch.empty(x.shape, dtype=torch.float32, device=dev) if y_fp32 else torch.empty_like(x)) if want_y else None
     codes = None
     if codes_kind == CODES_I8:
         codes = torch.empty(x.shape, dtype=torch.int8 if symmetric else torch.uint8, device=dev)
@@ -273,26 +275,31 @@ class AsymQuantizer(torch.autograd.Function):
         return ste_backward(grad_output, input, clip_val), None, None, None
 
 
+def lowbit_weight(weight: torch.Tensor, w_bits: int, layerwise: bool) -> torch.Tensor:
+    """The effective weight (q - w) + w of w_bits in {1, 2} (reference utils_quant.py:202-242)."""
+    _require_cuda(weight, "low-bit weight quant")
+    dt = _dtype_code(weight)
+    w = weight.detach()
+    w = w if w.is_contiguous() else w.contiguous()
+    out = torch.empty_like(w)
+    rows, cols = w.shape
+    L = _lib.lib()
+    ws_bytes = int(L.qat_lowbit_workspace_bytes(rows, int(bool(layerwise))))
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=w.device)
+    with _on(w.device):
+        rc = L.qat_lowbit_weight_fwd(w.data_ptr(), out.data_ptr(), rows, cols, dt, int(w_bits),
+                                     int(bool(layerwise)), _ptr(ws), ws_bytes, _stream_ptr(w.device))
+    check(rc, "qat_lowbit_weight_fwd")
+    return out
+
+
 class _LowBitWeight(torch.autograd.Function):
     """w_bits in {1, 2}: forward value (q - w) + w, identity gradient
     (reference utils_quant.py:202-242)."""
 
     @staticmethod
     def forward(ctx, weight, w_bits, layerwise):
-        _require_cuda(weight, "low-bit weight quant")
-        dt = _dtype_code(weight)
-        w = weight.detach()
-        w = w if w.is_contiguous() else w.contiguous()
-        out = torch.empty_like(w)
-        rows, cols = w.shape
-        L = _lib.lib()
-        ws_bytes = int(L.qat_lowbit_workspace_bytes(rows, int(bool(layerwise))))
-        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=w.device)
-        with _on(w.device):
-            rc = L.qat_lowbit_weight_fwd(w.data_ptr(), out.data_ptr(), rows, cols, dt, int(w_bits),
-                                         int(bool(layerwise)), _ptr(ws), ws_bytes, _stream_ptr(w.device))
-        check(rc, "qat_lowbit_weight_fwd")
-        return out
+        return lowbit_weight(weight, w_bits, layerwise)
 
     @staticmethod
     def backward(ctx, grad_output):
@@ -528,6 +535,144 @@ class _QuantLinearFn(torch.autograd.Function):
         return gx, gw, None, None, None
 
 
+# ------------------------------------------------------------------ the reference's operands on the own GEMM
+# QuantizeLinear off the int8 grid (reference utils_quant.py:190-254): 16-bit activations (W4-A16), weight-only
+# QAT (a_bits >= 32, W1/W2 included), activation-only (w_bits >= 32) and 9..31-bit weights.  Wider codes do not
+# suit kind::i8 (two MMAs per k-block for 16-bit codes, s32 overflow of the sum), so this route produces the
+# exact bf16 operands the reference hands F.linear and contracts them on qat_gemm_bf16, dgrad / wgrad with the
+# STE masks in the epilogue.  It differs from the reference only in the order of the fp32 accumulation.
+# Taken for modules that fuse_model marked (``_qat_operand_route``); the three kernel calls below are
+# module-level functions so that a CPU test can put torch statements in their place.
+def quant_operand(t: torch.Tensor, bits: int, amp: bool):
+    """(SymQuantizer's output as the bf16 operand of F.linear, packed STE mask for clip [-2, 2]).
+    Under autocast: the fp32 chain cast to bf16 in the same pass (QAT_BF16_AMP_CAST)."""
+    y, _, _, _, mask = fake_quant_forward(t, bits, False, True, mask_clip=(-2.0, 2.0), amp=amp, cast=amp)
+    return y, mask
+
+
+def lowbit_operand(w: torch.Tensor, bits: int) -> torch.Tensor:
+    """w_bits in {1, 2}: the effective weight; its gradient is the identity (no mask)."""
+    return lowbit_weight(w, bits, False)
+
+
+def gemm_bf16(a, b, mask, M: int, N: int, K: int, a_mn_major: int, b_mn_major: int,
+              cta_group: int = 0) -> torch.Tensor:
+    """out [M, N] bf16 = mask * (A . B^T) on qat_gemm_bf16 (layouts and cta_group: include/qat_b200.h)."""
+    out = torch.empty((M, N), dtype=torch.bfloat16, device=a.device)
+    with _on(a.device):
+        rc = _lib.lib().qat_gemm_bf16(a.data_ptr(), b.data_ptr(), out.data_ptr(), _ptr(mask), M, N, K,
+                                      a_mn_major, b_mn_major, QAT_BF16, cta_group, _stream_ptr(a.device))
+    check(rc, "qat_gemm_bf16")
+    return out
+
+
+def _route_device_ok(t: torch.Tensor) -> bool:
+    """The route's kernels exist for CUDA tensors only (a CPU test patches this with emulated kernels)."""
+    return t.is_cuda
+
+
+def _stream_key(dev) -> int:
+    return _stream_ptr(dev) if dev.type == "cuda" else 0
+
+
+def operand_route_config(lin) -> bool:
+    """The module configurations the operand route serves: symmetric, no layerwise flag, at least one operand
+    quantized, both feature counts multiples of 8 (TMA pitch), and not on the int8 grid."""
+    w, a = lin.w_bits, lin.a_bits
+    quant_x = 2 < a < 32
+    return (isinstance(lin, QuantizeLinear)
+            and (quant_x or w < 32) and w >= 1
+            and not (3 <= w <= 8 and 3 <= a <= 8)
+            and (not quant_x or getattr(lin, "act_quantizer", None) is SymQuantizer)
+            and not lin.act_layerwise and not lin.weight_layerwise
+            and lin.in_features % 8 == 0 and lin.out_features % 8 == 0)
+
+
+class _OperandLinearFn(torch.autograd.Function):
+    """out = x_op . W_op^T with the reference's bf16 operands (see the section comment).
+
+    forward : K1 writes each quantized operand (+ its packed STE mask); W1/W2 weights come from the low-bit
+              kernel; an unquantized operand is the tensor itself.  The weight operand is kept for the
+              checkpoint recompute like _QuantLinearFn's codes (QAT_B200_CACHE, QAT_B200_WEIGHT_REUSE) and the
+              activation operand is shared through the activation slot (q/k/v, gate/up).
+    backward: gx = mask_x * (g . W_op), gw = mask_w * (g^T . x_op), both on qat_gemm_bf16.
+    """
+
+    @staticmethod
+    def forward(ctx, input, weight, w_bits, a_bits, owner):
+        K = input.shape[-1]
+        N = weight.shape[0]
+        x2 = input.detach().reshape(-1, K)
+        if not x2.is_contiguous():
+            x2 = x2.contiguous()
+        w = weight.detach()
+        if not w.is_contiguous():
+            w = w.contiguous()
+        T = x2.shape[0]
+        dev = x2.device
+        amp = torch.is_autocast_enabled("cuda")
+        stream = _stream_key(dev)
+        mode = _cache_mode()
+
+        if 2 < a_bits < 32:
+            xkey = ("operand", x2.data_ptr(), input._version, T, K, amp, a_bits, stream)
+            slot = _ACT_SLOT.get(dev.index) if mode else None
+            if slot is not None and slot[0] == xkey and slot[3]() is input:
+                xq, xm = slot[2]
+            else:
+                xq, xm = quant_operand(x2, a_bits, amp)
+            if mode:
+                _ACT_SLOT[dev.index] = (xkey, None, (xq, xm), weakref.ref(input))
+        else:
+            xq, xm = x2, None
+
+        if w_bits < 32:
+            wkey = ("operand", w.data_ptr(), weight._version, N, K, amp, w_bits, stream)
+            cached = None
+            if owner is not None and (mode == 2 or (mode == 1 and _in_backward_pass())):
+                cached = getattr(owner, "_qat_wfeed", None)
+            if cached is not None and cached[0] == wkey:
+                wq, wm = cached[1]
+            elif w_bits >= 3:
+                wq, wm = quant_operand(w, w_bits, amp)
+            else:
+                wq, wm = lowbit_operand(w, w_bits), None
+            if mode:
+                if owner is not None and _weight_reuse_enabled() and (mode == 2 or owner.training):
+                    owner._qat_wfeed = (wkey, (wq, wm))
+                elif owner is not None and getattr(owner, "_qat_wfeed", None) is not None:
+                    owner._qat_wfeed = None
+        else:
+            wq, wm = w, None
+
+        out = gemm_bf16(xq, wq, None, T, N, K, 0, 0)
+        ctx.save_for_backward(xq, wq, xm, wm)
+        ctx.owner_ref = weakref.ref(owner) if (owner is not None and mode == 1) else None
+        ctx.dims = (T, N, K)
+        ctx.in_shape = input.shape
+        return out.view(*input.shape[:-1], N)
+
+    @staticmethod
+    def backward(ctx, grad_output):
+        xq, wq, xm, wm = ctx.saved_tensors
+        T, N, K = ctx.dims
+        g2 = grad_output.reshape(T, N)
+        if g2.dtype != torch.bfloat16:
+            g2 = g2.to(torch.bfloat16)
+        if not g2.is_contiguous() or g2.data_ptr() % 16:
+            g2 = g2.contiguous() if not g2.is_contiguous() else g2.clone()
+        gx = gw = None
+        if ctx.needs_input_grad[0]:
+            gx = gemm_bf16(g2, wq, xm, T, K, N, 0, 1).view(ctx.in_shape)
+        if ctx.needs_input_grad[1]:
+            gw = gemm_bf16(g2, xq, wm, N, K, T, 1, 1)
+        owner = ctx.owner_ref() if ctx.owner_ref is not None else None
+        if owner is not None:
+            owner._qat_wfeed = None
+        _ACT_SLOT.pop(g2.device.index, None)
+        return gx, gw, None, None, None
+
+
 def dequant_codes(codes, row_e, dtype):
     """out[r, c] = codes[r, c] / row_e[r] in ``dtype`` (exact IEEE quotient, one rounding)."""
     rows, cols = codes.shape
@@ -598,12 +743,30 @@ class QuantizeLinear(nn.Linear):
             and not (torch.is_autocast_enabled("cuda") and torch.get_autocast_dtype("cuda") != input_.dtype)
         )
 
+    def _can_route(self, input_: torch.Tensor) -> bool:
+        """The operand route (_OperandLinearFn): modules fuse_model marked, bf16 CUDA operands."""
+        return (
+            self.__dict__.get("_qat_operand_route", False)
+            and operand_route_config(self)
+            and _route_device_ok(input_)
+            and input_.device == self.weight.device
+            and input_.dtype == torch.bfloat16
+            and self.weight.dtype == torch.bfloat16
+            and 1 <= input_.dim() <= 3
+            and input_.numel() > 0
+            and input_.shape[-1] == self.weight.shape[1]
+            and input_.data_ptr() % 16 == 0 and self.weight.data_ptr() % 16 == 0
+            and not (torch.is_autocast_enabled("cuda") and torch.get_autocast_dtype("cuda") != torch.bfloat16)
+        )
+
     def forward(self, input_):
         assert len(self.weight.size()) == 2
         real_weights = self.weight
 
         if self._can_fuse(input_):
             return _QuantLinearFn.apply(input_, real_weights, self.w_bits, self.a_bits, self)
+        if self._can_route(input_):
+            return _OperandLinearFn.apply(input_, real_weights, self.w_bits, self.a_bits, self)
 
         if self.w_bits >= 32:
             weight = self.weight
