@@ -219,17 +219,6 @@ int qat_dequant_codes(const int8_t* codes, const float* row_e, void* out, int64_
  */
 int qat_gemm_bf16(const void* a, const void* b, void* out, const uint8_t* mask, int64_t M, int64_t N,
                   int64_t K, int a_mn_major, int b_mn_major, int out_dtype, int cta_group, void* stream);
-/*
- * The same contraction with B given as what the forward kept — int8 codes [K, N] (the rows of B are the
- * contraction index: W's codes [N_out, K_in] for dgrad, x's codes [T, K_in] for wgrad) and one divisor per
- * row, b_row_e [K].  Converter warps rebuild each 64 x 256 tile of fl_bf16(code / e[row]) in shared memory
- * (bit-identical to qat_dequant_codes) while the tensor core works on the previous tiles, so the operand is
- * never written to HBM.  N % 16 == 0.
- */
-int qat_gemm_bf16_codes(const void* a, const int8_t* b_codes, const float* b_row_e, void* out, const uint8_t* mask,
-                        int64_t M, int64_t N, int64_t K, int a_mn_major, int out_dtype, int cta_group, void* stream);
-/* Test hook: override the MN-major descriptor strides (bytes); 0, 0 restores the canonical ones. */
-int qat_gemm_bf16_debug_strides(uint32_t lbo_bytes, uint32_t sbo_bytes);
 
 /*
  * Fused causal attention on tcgen05 — replaces the eager block of

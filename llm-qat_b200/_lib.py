@@ -55,9 +55,6 @@ def _declare(lib):
         "qat_dequant_codes": (I, [P, P, P, L, L, I, P]),
         # a, b, out, mask, M, N, K, a_mn, b_mn, out_dtype, cta_group, stream
         "qat_gemm_bf16": (I, [P, P, P, P, L, L, L, I, I, I, I, P]),
-        "qat_gemm_bf16_debug_strides": (I, [ctypes.c_uint32, ctypes.c_uint32]),
-        # a, b_codes, b_row_e, out, mask, M, N, K, a_mn, out_dtype, cta_group, stream
-        "qat_gemm_bf16_codes": (I, [P, P, P, P, P, L, L, L, I, I, I, P]),
         # q, k, v, o, lse, B, S, H, D, scale, causal, stream
         "qat_attn_fwd": (I, [P, P, P, P, P, I, I, I, I, F, I, P]),
         # q, k, v, o, do, lse, delta, dq, dk, dv, B, S, H, D, scale, causal, stream

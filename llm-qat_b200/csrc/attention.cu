@@ -29,7 +29,6 @@
 // (MUFU, 16 ex2 per clock) in the forward, shared-memory operand bandwidth of the N = 64 MMAs in the backward.
 #define QAT_PDL_FAMILY 6   // bit of QAT_B200_PDL_MASK (common.cuh)
 #include <cmath>
-#include <cstdlib>
 
 #include "umma.cuh"
 
@@ -85,7 +84,6 @@ struct AttnParams {
   int B, S, H;
   float scale;         // 1 / sqrt(D)
   int causal;
-  int pingpong;        // fwd: the two softmax warpgroups take turns at the exponentials (QAT_B200_ATTN_PINGPONG, default 1)
 };
 
 // =============================================================================================
@@ -250,7 +248,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant
     const bool tr = (threadIdx.x == 64 || threadIdx.x == 192);
     // exp token: warpgroup 0 goes first (warpgroup 1 hands it the token up front); the turns alternate strictly
     // — tile 0, 1, 2, ... — which is also the order the S tiles are produced in
-    const bool pingpong = p.pingpong != 0 && n_kv > 1;
+    const bool pingpong = n_kv > 1;
     if (pingpong && wg == 1) named_bar_arrive(2, 256);
     for (int j = wg; j < n_kv; j += 2, ++uses) {
       const uint32_t ph = (uint32_t)(uses & 1);
@@ -949,11 +947,6 @@ extern "C" int qat_attn_fwd(const void* q, const void* k, const void* v, void* o
   p.H = H;
   p.scale = softmax_scale;
   p.causal = causal ? 1 : 0;
-  static const int pingpong = [] {
-    const char* e = getenv("QAT_B200_ATTN_PINGPONG");
-    return (e && e[0] == '0') ? 0 : 1;
-  }();
-  p.pingpong = pingpong;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const dim3 grid((unsigned)((S + BM - 1) / BM), (unsigned)H, (unsigned)B);
   cudaError_t e = launch_pdl(attn_fwd_kernel, grid, dim3(fwd::kThreads), fwd::kSmem, st, mq, mk, mv, p);

@@ -6,7 +6,6 @@
 // the forward can save 1 B/elem of codes instead of the reference's two
 // dequantized tensors.  HBM-bound: 1 + sizeof(T) bytes per element.
 #define QAT_PDL_FAMILY 2   // bit of QAT_B200_PDL_MASK (common.cuh)
-#include <cstdlib>
 #include <type_traits>
 
 #include "common.cuh"
@@ -17,7 +16,7 @@ namespace {
 constexpr int kThreads = 256;
 
 // Tile = kThreads * unroll code groups, all loaded before use; ONE CTA PER TILE (no grid-stride cap).  Measured
-// (tests/gpu_dequant_tune.py, profiles/r02_dequant_ste_tune.json): the former cap of 8 CTAs per SM assumed an
+// (profiles/r02_dequant_ste_tune.json): the former cap of 8 CTAs per SM assumed an
 // occupancy the 40-64 register kernels do not have (5-6 CTAs per SM), so a second, ragged wave of CTAs each
 // walked 4-5 tiles on a third of the slots: 0.77 of the HBM peak at [11008, 4096]; uncapped, the block scheduler
 // balances tile by tile: 0.85.  Large tensors take 8 groups per thread (fp32 divisors: 26.7 -> 24.7 us), small
@@ -131,18 +130,9 @@ extern "C" int qat_dequant_codes(const int8_t* codes, const float* row_e, void* 
   const int per = dtype == QAT_BF16 ? 8 : 4;    // codes per thread-iteration == one 16-byte store
   const int64_t ngroups = rows * cols / per;
   QAT_CHECK_ARG(cols / per < (1ll << 31), "row too long");
-  // tile shape / grid cap: fixed defaults; QAT_B200_DEQUANT_TUNE=1 re-reads QAT_B200_DEQUANT_UNROLL (2|4|8) and
-  // QAT_B200_DEQUANT_CTAS (CTAs per SM, 0 = one CTA per tile) on every call (tests/gpu_dequant_tune.py)
-  int unroll = ngroups >= kLargeGroups ? 8 : 2, ctas = kCtasPerSmDefault;
-  static const bool tune = [] { const char* e = getenv("QAT_B200_DEQUANT_TUNE"); return e != nullptr && e[0] == '1'; }();
-  if (tune) {
-    if (const char* e = getenv("QAT_B200_DEQUANT_UNROLL")) unroll = atoi(e);
-    if (const char* e = getenv("QAT_B200_DEQUANT_CTAS")) ctas = atoi(e);
-    QAT_CHECK_ARG(unroll == 2 || unroll == 4 || unroll == 8, "QAT_B200_DEQUANT_UNROLL must be 2, 4 or 8");
-    QAT_CHECK_ARG(ctas >= 0 && ctas <= 64, "QAT_B200_DEQUANT_CTAS must be in [0, 64]");
-  }
+  const int unroll = ngroups >= kLargeGroups ? 8 : 2;
   int64_t grid = (ngroups + kThreads * unroll - 1) / (kThreads * unroll);
-  const int64_t cap = ctas > 0 ? (int64_t)num_sms() * ctas : (int64_t)0x7fffffff;
+  const int64_t cap = kCtasPerSmDefault > 0 ? (int64_t)num_sms() * kCtasPerSmDefault : (int64_t)0x7fffffff;
   if (grid > cap) grid = cap;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const bool idx32 = ngroups < (1ll << 32);
@@ -165,11 +155,10 @@ extern "C" int qat_dequant_codes(const int8_t* codes, const float* row_e, void* 
   const dim3 g((unsigned)grid), b(kThreads);
 #define QAT_DEQUANT_LAUNCH(DT, IDX, U) \
   (void)launch_pdl(dequant_codes_kernel<DT, IDX, U>, g, b, 0, st, codes, row_e, out, ngroups, gpr, magic)
-#define QAT_DEQUANT_UNROLL(DT, IDX)                      \
-  do {                                                   \
-    if (unroll == 2) QAT_DEQUANT_LAUNCH(DT, IDX, 2);      \
-    else if (unroll == 8) QAT_DEQUANT_LAUNCH(DT, IDX, 8); \
-    else QAT_DEQUANT_LAUNCH(DT, IDX, 4);                  \
+#define QAT_DEQUANT_UNROLL(DT, IDX)                 \
+  do {                                              \
+    if (unroll == 8) QAT_DEQUANT_LAUNCH(DT, IDX, 8); \
+    else QAT_DEQUANT_LAUNCH(DT, IDX, 2);             \
   } while (0)
   if (dtype == QAT_BF16) {
     if (idx32) QAT_DEQUANT_UNROLL(QAT_BF16, true);

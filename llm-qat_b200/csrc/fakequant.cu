@@ -726,16 +726,6 @@ constexpr int kMaxGroup = 1024;
 
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
-// tuning knob (development): QAT_B200_MAX_ITERS=1..8 caps the vectors per thread
-int tuned_max_iters() {
-  static int v = [] {
-    const char* e = getenv("QAT_B200_MAX_ITERS");
-    int n = e ? atoi(e) : kMaxIters;
-    return (n >= 1 && n <= kMaxIters) ? n : kMaxIters;
-  }();
-  return v;
-}
-
 struct Plan {
   bool vec;
   bool fused;  // row fits registers
@@ -754,12 +744,11 @@ Plan make_plan(const void* x, const void* y, int64_t rows, int64_t cols, int dty
   // fixed work (reduction tree, scale broadcast, addressing) is ~200 instructions,
   // so prefer many vectors per thread; among candidates take the one with the
   // fewest idle vector slots, ties to the smaller group.
-  const int max_iters = tuned_max_iters();
   int best_group = 0;
   int64_t best_iters = 0, best_slots = 0;
   for (int group = 32; group <= kMaxGroup; group <<= 1) {
     const int64_t iters = (pl.nvec + group - 1) / group;
-    if (iters > max_iters) continue;
+    if (iters > kMaxIters) continue;
     const int64_t slots = iters * group;
     if (best_group == 0 || slots < best_slots) {
       best_group = group;
@@ -966,7 +955,7 @@ size_t qat_fwd_workspace_bytes(int64_t rows, int64_t cols, int dtype) {
   (void)dtype;
   // the scalar path may be chosen at run time when a pointer is misaligned, so
   // size for it: fused iff cols <= kMaxGroup * kMaxIters elements.
-  if (cols <= (int64_t)qat::kMaxGroup * qat::tuned_max_iters()) return 0;
+  if (cols <= (int64_t)qat::kMaxGroup * qat::kMaxIters) return 0;
   return (size_t)rows * 16;
 }
 

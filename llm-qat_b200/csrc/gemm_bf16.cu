@@ -39,35 +39,26 @@ constexpr int kEpiWarp0 = 4;
 constexpr int kEpiWarps = 4;
 constexpr uint32_t kChunkBytes = 64 * BLOCK_K * 2;   // one MN-major TMA box: 64 K-rows x 128 B = 8 KB
 
-// CODES: the B operand arrives as int8 codes + one divisor per contraction row and is turned into the
-// fake-quantized bf16 values inside the kernel (converter warps), see gemm_bf16_kernel.
-template <int CG, bool CODES = false>
+template <int CG>
 struct Cfg {
-  static constexpr int kStages = CODES ? (CG == 1 ? 3 : 5) : (CG == 1 ? 4 : 6);
+  static constexpr int kStages = CG == 1 ? 4 : 6;
   static constexpr int kTileM = BLOCK_M * CG;
   static constexpr int kBRows = BLOCK_N / CG;                     // B rows (N) staged by each CTA
   static constexpr uint32_t kABytes = BLOCK_M * BLOCK_K * 2;      // 16 KB
   static constexpr uint32_t kBBytes = kBRows * BLOCK_K * 2;       // 32 KB | 16 KB
-  static constexpr uint32_t kRawBytes = CODES ? kBRows * BLOCK_K : 0;   // int8 codes [64 rows][kBRows]: 16 KB | 8 KB
-  static constexpr uint32_t kStageBytes = kABytes + kBBytes + kRawBytes;
+  static constexpr uint32_t kStageBytes = kABytes + kBBytes;
   static __host__ __device__ constexpr uint32_t a(int s) { return (uint32_t)s * kStageBytes; }
   static __host__ __device__ constexpr uint32_t b(int s) { return (uint32_t)s * kStageBytes + kABytes; }
-  static __host__ __device__ constexpr uint32_t raw(int s) { return (uint32_t)s * kStageBytes + kABytes + kBBytes; }
   static constexpr uint32_t bars = kStages * kStageBytes;
   static __host__ __device__ constexpr uint32_t full(int s) { return bars + 8u * s; }
   static __host__ __device__ constexpr uint32_t empty(int s) { return bars + 8u * (kStages + s); }
-  static __host__ __device__ constexpr uint32_t rawfull(int s) { return bars + 8u * (2 * kStages + s); }   // CODES only
-  static __host__ __device__ constexpr uint32_t cvt(int s) { return bars + 8u * (3 * kStages + s); }       // CODES only
-  static __host__ __device__ constexpr uint32_t tfull(int a) { return bars + 8u * (4 * kStages + a); }
-  static __host__ __device__ constexpr uint32_t tempty(int a) { return bars + 8u * (4 * kStages + kAccStages + a); }
-  static constexpr uint32_t tmem_ptr = bars + 8u * (4 * kStages + 2 * kAccStages);
+  static __host__ __device__ constexpr uint32_t tfull(int a) { return bars + 8u * (2 * kStages + a); }
+  static __host__ __device__ constexpr uint32_t tempty(int a) { return bars + 8u * (2 * kStages + kAccStages + a); }
+  static constexpr uint32_t tmem_ptr = bars + 8u * (2 * kStages + 2 * kAccStages);
   static constexpr uint32_t total = tmem_ptr + 16;
   static constexpr uint32_t kSmemBytes = total + 1024;
 };
 static_assert(Cfg<1>::kSmemBytes <= 232448 && Cfg<2>::kSmemBytes <= 232448, "over the 227 KB per-CTA limit");
-static_assert(Cfg<1, true>::kSmemBytes <= 232448 && Cfg<2, true>::kSmemBytes <= 232448, "over the 227 KB per-CTA limit");
-constexpr int kCvtWarp0 = 8;      // CODES: warps 8..15 convert
-constexpr int kCvtWarps = 8;
 
 struct Params {
   void* out;             // [M, N] row-major, bf16 or fp32
@@ -75,28 +66,7 @@ struct Params {
   int64_t M, N, K;
   int out_dtype;
   int m_blocks, n_blocks, k_blocks;
-  uint32_t lbo_a, sbo_a, lbo_b, sbo_b;   // MN-major descriptor strides (bytes)
-  const float* b_row_e;                  // CODES: divisor of each contraction row of B, [K]
 };
-
-// 8 int8 codes / e -> 8 bf16: the arithmetic of dequant_codes_kernel (dequant.cu), so that the operand the
-// tensor core sees is bit-identical to the tensor that kernel would have written
-__device__ __forceinline__ uint4 dequant8(uint32_t lo, uint32_t hi, float e, float r, bool mulq, bool fast) {
-  float y[8];
-#pragma unroll
-  for (int k = 0; k < 8; ++k) y[k] = (float)(int)(int8_t)(((k < 4 ? lo : hi) >> (8 * (k & 3))) & 0xffu);
-  if (mulq) {
-#pragma unroll
-    for (int k = 0; k < 8; ++k) y[k] = __fmul_rn(y[k], r);
-  } else if (fast) {
-#pragma unroll
-    for (int k = 0; k < 8; ++k) y[k] = div_code_by_recip(y[k], e, r);
-  } else {
-#pragma unroll
-    for (int k = 0; k < 8; ++k) y[k] = __fdiv_rn(y[k], e);
-  }
-  return make_uint4(pack_bf16x2(y[0], y[1]), pack_bf16x2(y[2], y[3]), pack_bf16x2(y[4], y[5]), pack_bf16x2(y[6], y[7]));
-}
 
 // 32 consecutive mask bits starting at flat element index i0 (any alignment)
 __device__ __forceinline__ uint32_t mask_bits32(const uint8_t* mask, int64_t i0, int64_t nbytes) {
@@ -155,15 +125,11 @@ __device__ __forceinline__ void tma_any(uint32_t dst, const CUtensorMap* map, ui
   if (CG == 1) tma_load_2d(dst, map, bar, c0, c1); else tma_load_2d_pair(dst, map, bar, c0, c1);
 }
 
-// B_MODE: 0 = bf16 K-major, 1 = bf16 MN-major, 2 = int8 codes [K, N] + row divisors, converted to the MN-major
-// bf16 tile in shared memory by warps 8..15 while the tensor core works on the previous k-blocks.
-template <bool A_MN, int B_MODE, int CG>
-__global__ void __launch_bounds__(B_MODE == 2 ? 512 : kThreads, 1)
+template <bool A_MN, bool B_MN, int CG>
+__global__ void __launch_bounds__(kThreads, 1)
 gemm_bf16_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
                  const Params p) {
-  constexpr bool B_MN = B_MODE != 0;
-  constexpr bool CODES = B_MODE == 2;
-  using C = Cfg<CG, CODES>;
+  using C = Cfg<CG>;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* base_ptr = smem_raw + (base - smem_u32(smem_raw));
@@ -182,10 +148,6 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
     for (int s = 0; s < C::kStages; ++s) {
       mbar_init(base + C::full(s), 1);
       mbar_init(base + C::empty(s), 1);
-      if (CODES) {
-        mbar_init(base + C::rawfull(s), 1);            // this CTA's own code tile has landed
-        mbar_init(base + C::cvt(s), CG * kCvtWarps);   // every converter warp of every CTA of the pair
-      }
     }
 #pragma unroll
     for (int a = 0; a < kAccStages; ++a) {
@@ -216,9 +178,8 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
         for (int kb = 0; kb < p.k_blocks; ++kb) {
           mbar_wait(base + C::empty(stage), phase ^ 1u);
           const uint32_t full = base + C::full(stage);
-          constexpr uint32_t kFullBytes = CODES ? C::kABytes : C::kStageBytes;   // CODES: B arrives via rawfull / cvt
-          if (CG == 1) mbar_expect_tx(full, kFullBytes);
-          else if (rank == 0) mbar_expect_tx(full, 2 * kFullBytes);
+          if (CG == 1) mbar_expect_tx(full, C::kStageBytes);
+          else if (rank == 0) mbar_expect_tx(full, 2 * C::kStageBytes);
           const int32_t k0 = kb * BLOCK_K;
           if (!A_MN) {
             tma_any<CG>(base + C::a(stage), &map_a, full, k0, a_row);              // box {64 k, 128 m}
@@ -227,12 +188,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
             for (int c = 0; c < BLOCK_M / 64; ++c)                                 // boxes {64 m, 64 k}
               tma_any<CG>(base + C::a(stage) + c * kChunkBytes, &map_a, full, a_row + 64 * c, k0);
           }
-          if (CODES) {
-            // int8 codes [K, N]: one un-swizzled box {kBRows bytes of N, 64 rows of K}, completing on THIS
-            // CTA's barrier (its own converter warps consume it)
-            mbar_expect_tx(base + C::rawfull(stage), C::kRawBytes);
-            tma_load_2d(base + C::raw(stage), &map_b, base + C::rawfull(stage), b_row, k0);
-          } else if (!B_MN) {
+          if (!B_MN) {
             tma_any<CG>(base + C::b(stage), &map_b, full, k0, b_row);              // box {64 k, kBRows n}
           } else {
 #pragma unroll
@@ -258,11 +214,10 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
         const uint32_t tmem_d = tmem_base + (uint32_t)(acc * BLOCK_N);
         for (int kb = 0; kb < p.k_blocks; ++kb) {
           mbar_wait(base + C::full(stage), phase);
-          if (CODES) mbar_wait(base + C::cvt(stage), phase);
           tcgen05_fence_after();
-          const uint64_t adesc = A_MN ? make_smem_desc_mn(base + C::a(stage), p.lbo_a, p.sbo_a)
+          const uint64_t adesc = A_MN ? make_smem_desc_mn(base + C::a(stage), kChunkBytes, 1024u)
                                       : make_smem_desc(base + C::a(stage));
-          const uint64_t bdesc = B_MN ? make_smem_desc_mn(base + C::b(stage), p.lbo_b, p.sbo_b)
+          const uint64_t bdesc = B_MN ? make_smem_desc_mn(base + C::b(stage), kChunkBytes, 1024u)
                                       : make_smem_desc(base + C::b(stage));
           // per UMMA_K = 16 elements: K-major +32 B inside the swizzle row; MN-major +16 rows = 2048 B
           constexpr uint64_t a_step = A_MN ? (16u * 128u) >> 4 : 2u;
@@ -280,49 +235,6 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
         if (++acc == kAccStages) {
           acc = 0;
           acc_phase ^= 1u;
-        }
-      }
-    }
-  } else if (CODES && warp >= kCvtWarp0) {
-    // ===================== converters: int8 codes -> fake-quantized bf16, MN-major swizzled tile =====================
-    // 256 threads per k-block: thread t owns row r = t / 4 of the 64 contraction rows and a quarter of the
-    // kBRows columns (32 or 64 codes); out(r, n) = fl_bf16(code / e[r]) exactly as dequant_codes_kernel.
-    const int t = threadIdx.x - kCvtWarp0 * 32;
-    const int r = t >> 2, qd = t & 3;
-    constexpr int kPer = C::kBRows / 4;            // codes per thread: 64 (CG 1) | 32 (CG 2)
-    int stage = 0;
-    uint32_t phase = 0;
-    for (int tile = unit; tile < num_tiles; tile += num_units) {
-      for (int kb = 0; kb < p.k_blocks; ++kb) {
-        const int64_t krow = (int64_t)kb * BLOCK_K + r;
-        const float e = krow < p.K ? __ldg(p.b_row_e + krow) : 1.0f;
-        const bool fast = recip_range_ok(e);
-        const float rcp = __frcp_rn(e);
-        const bool mulq = fast && Num<QAT_BF16>::fl(e) == e;
-        mbar_wait(base + C::rawfull(stage), phase);
-        const uint32_t src = base + C::raw(stage) + (uint32_t)(r * C::kBRows + qd * kPer);
-#pragma unroll
-        for (int i = 0; i < kPer / 16; ++i) {
-          uint32_t c0, c1, c2, c3;
-          asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(c0), "=r"(c1), "=r"(c2), "=r"(c3) : "r"(src + 16u * i));
-          const int n0 = qd * kPer + i * 16;       // first of these 16 columns inside the CTA's kBRows
-#pragma unroll
-          for (int hlf = 0; hlf < 2; ++hlf) {
-            const int n = n0 + hlf * 8;
-            const uint4 v = dequant8(hlf ? c2 : c0, hlf ? c3 : c1, e, rcp, mulq, fast);
-            const uint32_t dst = base + C::b(stage) + (uint32_t)(n >> 6) * kChunkBytes + (uint32_t)r * 128u +
-                                 ((((uint32_t)(n >> 3) & 7u) ^ ((uint32_t)r & 7u)) << 4);
-            asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(dst), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-          }
-        }
-        fence_proxy_async_smem();
-        __syncwarp();
-        if (lane == 0) {
-          if (CG == 1) mbar_arrive(base + C::cvt(stage)); else mbar_arrive_remote(base + C::cvt(stage), 0u);
-        }
-        if (++stage == C::kStages) {
-          stage = 0;
-          phase ^= 1u;
         }
       }
     }
@@ -367,14 +279,14 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
   }
 }
 
-template <bool A_MN, int B_MODE, int CG>
+template <bool A_MN, bool B_MN, int CG>
 int launch(const CUtensorMap& ma, const CUtensorMap& mb, const Params& p, cudaStream_t st) {
-  using C = Cfg<CG, B_MODE == 2>;
+  using C = Cfg<CG>;
   static bool attr_set[64] = {};
   int dev = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) dev = 0;
   if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(gemm_bf16_kernel<A_MN, B_MODE, CG>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    cudaError_t e = cudaFuncSetAttribute(gemm_bf16_kernel<A_MN, B_MN, CG>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)C::kSmemBytes);
     if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(gemm_bf16_kernel)");
     if (dev >= 0 && dev < 64) attr_set[dev] = true;
@@ -384,7 +296,7 @@ int launch(const CUtensorMap& ma, const CUtensorMap& mb, const Params& p, cudaSt
   if (units > tiles) units = tiles;
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3((unsigned)(units * CG));
-  cfg.blockDim = dim3(B_MODE == 2 ? 512 : kThreads);
+  cfg.blockDim = dim3(kThreads);
   cfg.dynamicSmemBytes = C::kSmemBytes;
   cfg.stream = st;
   cudaLaunchAttribute attr[2];
@@ -396,7 +308,7 @@ int launch(const CUtensorMap& ma, const CUtensorMap& mb, const Params& p, cudaSt
   attr[1].val.programmaticStreamSerializationAllowed = pdl_enabled(QAT_PDL_FAMILY) ? 1 : 0;
   cfg.attrs = attr;
   cfg.numAttrs = 2;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, gemm_bf16_kernel<A_MN, B_MODE, CG>, ma, mb, p);
+  cudaError_t e = cudaLaunchKernelEx(&cfg, gemm_bf16_kernel<A_MN, B_MN, CG>, ma, mb, p);
   if (e != cudaSuccess) return cuda_fail(e, "gemm_bf16_kernel launch");
   QAT_CHECK_LAUNCH("gemm_bf16_kernel");
   return QAT_OK;
@@ -414,17 +326,8 @@ int pick_cg(int64_t M, int64_t N) {
   return pair_tiles >= num_sms() / 2 ? 2 : 1;
 }
 
-// debug overrides of the MN-major descriptor strides (tests/gpu_umma_probe.py): 0 = canonical
-uint32_t g_dbg_lbo = 0, g_dbg_sbo = 0;
-
 }  // namespace
 }  // namespace qat
-
-extern "C" int qat_gemm_bf16_debug_strides(uint32_t lbo_bytes, uint32_t sbo_bytes) {
-  qat::g_dbg_lbo = lbo_bytes;
-  qat::g_dbg_sbo = sbo_bytes;
-  return QAT_OK;
-}
 
 extern "C" int qat_gemm_bf16(const void* a, const void* b, void* out, const uint8_t* mask, int64_t M, int64_t N,
                              int64_t K, int a_mn_major, int b_mn_major, int out_dtype, int cta_group,
@@ -458,76 +361,16 @@ extern "C" int qat_gemm_bf16(const void* a, const void* b, void* out, const uint
   p.m_blocks = (int)((M + BLOCK_M * cg - 1) / (BLOCK_M * cg));
   p.n_blocks = (int)((N + BLOCK_N - 1) / BLOCK_N);
   p.k_blocks = (int)((K + BLOCK_K - 1) / BLOCK_K);
-  p.lbo_a = p.lbo_b = g_dbg_lbo ? g_dbg_lbo : kChunkBytes;
-  p.sbo_a = p.sbo_b = g_dbg_sbo ? g_dbg_sbo : 1024u;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   const int sel = (a_mn_major ? 4 : 0) | (b_mn_major ? 2 : 0) | (cg == 2 ? 1 : 0);
   switch (sel) {
-    case 0: return launch<false, 0, 1>(ma, mb, p, st);
-    case 1: return launch<false, 0, 2>(ma, mb, p, st);
-    case 2: return launch<false, 1, 1>(ma, mb, p, st);
-    case 3: return launch<false, 1, 2>(ma, mb, p, st);
-    case 4: return launch<true, 0, 1>(ma, mb, p, st);
-    case 5: return launch<true, 0, 2>(ma, mb, p, st);
-    case 6: return launch<true, 1, 1>(ma, mb, p, st);
-    default: return launch<true, 1, 2>(ma, mb, p, st);
+    case 0: return launch<false, false, 1>(ma, mb, p, st);
+    case 1: return launch<false, false, 2>(ma, mb, p, st);
+    case 2: return launch<false, true, 1>(ma, mb, p, st);
+    case 3: return launch<false, true, 2>(ma, mb, p, st);
+    case 4: return launch<true, false, 1>(ma, mb, p, st);
+    case 5: return launch<true, false, 2>(ma, mb, p, st);
+    case 6: return launch<true, true, 1>(ma, mb, p, st);
+    default: return launch<true, true, 2>(ma, mb, p, st);
   }
-}
-
-// B given as int8 codes [K, N] (row-major, what qat_sym_fwd's feed writes for a [K, N] tensor whose rows are
-// its reduction rows) and its row divisors e[K]: the contraction runs over the rows, so the per-row divisor
-// cannot move to the epilogue — the operand is rebuilt tile by tile inside the kernel instead.
-extern "C" int qat_gemm_bf16_codes(const void* a, const int8_t* b_codes, const float* b_row_e, void* out,
-                                   const uint8_t* mask, int64_t M, int64_t N, int64_t K, int a_mn_major,
-                                   int out_dtype, int cta_group, void* stream) {
-  using namespace qat;
-  QAT_CHECK_ARG(out_dtype == QAT_F32 || out_dtype == QAT_BF16, "out_dtype must be QAT_F32 or QAT_BF16");
-  QAT_CHECK_ARG(M >= 0 && N >= 0 && K > 0, "bad GEMM shape [%lld, %lld, %lld]", (long long)M, (long long)N,
-                (long long)K);
-  if (M == 0 || N == 0) return QAT_OK;
-  QAT_CHECK_ARG(a && b_codes && b_row_e && out, "NULL operand");
-  QAT_CHECK_ARG(((uintptr_t)a & 15) == 0 && ((uintptr_t)b_codes & 15) == 0 && ((uintptr_t)out & 15) == 0,
-                "operands must be 16-byte aligned");
-  QAT_CHECK_ARG(M < (1ll << 31) && N < (1ll << 31) && K < (1ll << 31), "dimension too large");
-  QAT_CHECK_ARG((a_mn_major ? M : K) % 8 == 0, "A's contiguous dimension must be a multiple of 8 elements");
-  QAT_CHECK_ARG(N % 16 == 0, "N must be a multiple of 16 (TMA pitch of the int8 codes)");
-  QAT_CHECK_ARG(cta_group == 0 || cta_group == 1 || cta_group == 2, "cta_group must be 0 (automatic), 1 or 2");
-  const int cg = cta_group ? cta_group : pick_cg(M, N);
-  CUtensorMap ma, mb;
-  int rc = a_mn_major ? make_map_bf16_2d(&ma, a, K, M, M, 64) : make_map_bf16_2d(&ma, a, M, K, K, BLOCK_M);
-  if (rc != QAT_OK) return rc;
-  {
-    EncodeFn enc = get_encode();
-    if (enc == nullptr) {
-      set_error("cuTensorMapEncodeTiled is not available from the CUDA driver");
-      return QAT_ERR_UNSUPPORTED;
-    }
-    cuuint64_t dims[2] = {(cuuint64_t)N, (cuuint64_t)K};
-    cuuint64_t strides[1] = {(cuuint64_t)N};
-    cuuint32_t box[2] = {(cuuint32_t)(BLOCK_N / cg), (cuuint32_t)BLOCK_K};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = enc(&mb, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<int8_t*>(b_codes), dims, strides, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) {
-      set_error("cuTensorMapEncodeTiled failed (CUresult %d) for int8 codes [%lld, %lld]", (int)r, (long long)K, (long long)N);
-      return QAT_ERR_BAD_ARG;
-    }
-  }
-  Params p{};
-  p.out = out;
-  p.mask = mask;
-  p.M = M;
-  p.N = N;
-  p.K = K;
-  p.out_dtype = out_dtype;
-  p.m_blocks = (int)((M + BLOCK_M * cg - 1) / (BLOCK_M * cg));
-  p.n_blocks = (int)((N + BLOCK_N - 1) / BLOCK_N);
-  p.k_blocks = (int)((K + BLOCK_K - 1) / BLOCK_K);
-  p.lbo_a = p.lbo_b = kChunkBytes;
-  p.sbo_a = p.sbo_b = 1024u;
-  p.b_row_e = b_row_e;
-  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  if (a_mn_major) return cg == 2 ? launch<true, 2, 2>(ma, mb, p, st) : launch<true, 2, 1>(ma, mb, p, st);
-  return cg == 2 ? launch<false, 2, 2>(ma, mb, p, st) : launch<false, 2, 1>(ma, mb, p, st);
 }

@@ -9,13 +9,12 @@
 // the B200 box, two concurrent copies in the SAME direction (x beside g) drop the
 // link from 41 to 33 GB/s per direction.  The
 // ceiling is the link itself: 47 GB/s per direction with both directions busy
-// (tests/gpu_pcie_probe.py); this pipeline sustains 42 (tests/gpu_e2e_probe.py, profiles/r02_e2e_sweep.json:
-// 7.75 ms per configs[1] step with round 1's schedule at 8 MB, 7.50 ms with the split schedule at 16 MB).
+// (tests/gpu_pcie_probe.py); this pipeline sustains 42 (profiles/r02_e2e_sweep.json: 7.75 ms per configs[1]
+// step with both inputs copied ahead of the kernels at 8 MB, 7.50 ms with the split schedule at 16 MB).
 // Everything is ordered
 // after prior work on the caller's stream and the caller's stream waits for the
 // last D2H, so stream semantics are those of a single asynchronous call.
 #define QAT_PDL_FAMILY 9   // bit of QAT_B200_PDL_MASK (common.cuh)
-#include <cstdlib>
 #include <vector>
 
 #include "common.cuh"
@@ -53,15 +52,7 @@ Pipe* get_pipe() {
   return &pipes.back();
 }
 
-// per tensor per chunk; QAT_B200_HOST_CHUNK_MB=1..64 overrides (tuning)
-int64_t target_chunk_bytes() {
-  static const int64_t v = [] {
-    const char* e = getenv("QAT_B200_HOST_CHUNK_MB");
-    const int mb = e ? atoi(e) : 0;
-    return (int64_t)((mb >= 1 && mb <= 64) ? mb : 16) << 20;
-  }();
-  return v;
-}
+constexpr int64_t kChunkBytes = 16ll << 20;   // per tensor per chunk
 
 template <bool SYM>
 int fwd_bwd_host(const void* x_host, const void* g_host, void* y_host, void* gx_host, float lo,
@@ -101,7 +92,7 @@ int fwd_bwd_host(const void* x_host, const void* g_host, void* y_host, void* gx_
   // 1/8, 1/4, 1/2 of that: the D2H direction idles while the first chunk goes
   // in, and the H2D direction while the last one comes out, so short end
   // chunks cut those two bubbles from ~0.3 ms to ~0.04 ms per call.
-  int64_t chunk_rows = target_chunk_bytes() / (row_bytes > 0 ? row_bytes : 1);
+  int64_t chunk_rows = kChunkBytes / (row_bytes > 0 ? row_bytes : 1);
   if (chunk_rows < 1) chunk_rows = 1;
   // keep chunk starts 16-byte aligned for any row pitch
   int64_t align_rows = 1;
@@ -144,11 +135,6 @@ int fwd_bwd_host(const void* x_host, const void* g_host, void* y_host, void* gx_
   // Within a chunk the forward needs x only: x goes in, K1/K2 runs and y starts its way back while g is still
   // going in; then K3 and gx.  The outbound direction so trails the inbound one by HALF a chunk (one tensor's
   // slice), which lets the copies be twice as long for the same pipeline granularity.
-  // QAT_B200_HOST_SCHEDULE=chunk: both inputs first, then both kernels, then both outputs (round 1's order).
-  static const bool split = [] {
-    const char* e = getenv("QAT_B200_HOST_SCHEDULE");
-    return !(e && e[0] == 'c');
-  }();
   cudaStream_t s_in = pipe->in, s_out = pipe->out;
   const char* src[2] = {reinterpret_cast<const char*>(x_host), reinterpret_cast<const char*>(g_host)};
   char* dst_dev[2] = {dx, dg};
@@ -182,13 +168,11 @@ int fwd_bwd_host(const void* x_host, const void* g_host, void* y_host, void* gx_
     };
     int rc;
     QAT_TRY(copy_in(0));
-    if (bwd && !split) QAT_TRY(copy_in(1));
     if ((rc = forward()) != QAT_OK) return rc;
-    if (!bwd || split) QAT_TRY(copy_out(0));
+    QAT_TRY(copy_out(0));
     if (bwd) {
-      if (split) QAT_TRY(copy_in(1));
+      QAT_TRY(copy_in(1));
       if ((rc = qat_ste_bwd(dg + off, dx + off, dgx + off, nullptr, lo, hi, nr * cols, dtype, st)) != QAT_OK) return rc;
-      if (!split) QAT_TRY(copy_out(0));
       QAT_TRY(copy_out(1));
     }
   }

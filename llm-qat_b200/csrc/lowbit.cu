@@ -15,7 +15,6 @@
 #define QAT_PDL_FAMILY 3   // bit of QAT_B200_PDL_MASK (common.cuh)
 #include <algorithm>
 #include <atomic>
-#include <cstdlib>
 #include <type_traits>
 
 #include "common.cuh"
@@ -285,13 +284,9 @@ bool launch_exact(const void* w, void* out, int64_t rows, int64_t cols, int w_bi
   const size_t smem = exact_smem_bytes(cols, eb, &gs_offset);
   if (smem > kMaxDynSmem || rows > 0x7fffffffLL || cols >= (1LL << 24)) return false;
   // one round of four 16-byte loads per thread where the row allows it: a CTA's lifetime is what the last,
-  // partly filled wave of rows costs, so it is kept short rather than the CTA small
+  // partly filled wave of rows costs, so it is kept short rather than the CTA small (profiles/r02_lowbit_exact.json)
   const int64_t chunks = ((int64_t)cols * eb + 15) / 16;
-  int threads = (int)std::min<int64_t>(512, std::max<int64_t>(128, ((chunks + 3) / 4 + 63) / 64 * 64));
-  if (const char* t = getenv("QAT_B200_LOWBIT_THREADS")) {   // tuning knob (tests/gpu_lowbit_probe.py)
-    const int v = atoi(t);
-    if (v >= 32 && v <= 512 && v % 32 == 0) threads = v;
-  }
+  const int threads = (int)std::min<int64_t>(512, std::max<int64_t>(128, ((chunks + 3) / 4 + 63) / 64 * 64));
   const bool vec = ((uintptr_t)w & 15) == 0 && ((uintptr_t)out & 15) == 0;
   *err = vec ? launch_exact_variant<DT, true>(w, out, rows, cols, w_bits, smem, gs_offset, threads, st)
              : launch_exact_variant<DT, false>(w, out, rows, cols, w_bits, smem, gs_offset, threads, st);

@@ -6,7 +6,6 @@
 // streaming pass: read g, read x (or a forward-emitted packed mask), write gx.
 // HBM-bound: 3*sizeof(T) B/elem from x, 2*sizeof(T) + 1/8 B/elem from a mask.
 #define QAT_PDL_FAMILY 1   // bit of QAT_B200_PDL_MASK (common.cuh)
-#include <cstdlib>
 #include "common.cuh"
 
 namespace qat {
@@ -18,7 +17,7 @@ constexpr int kUnroll = 4;  // 16-byte vectors per thread per tile, all loaded b
 // Grid of the vector kernel: ONE CTA PER TILE (0 = no cap).  The former cap of 8 CTAs per SM assumed an occupancy
 // the 48-register bf16 kernel does not have (5 per SM), leaving a ragged second wave of grid-striding CTAs:
 // bf16 [8192, 4096] 35.1 -> 33.1 us (0.89 -> 0.94 of the HBM peak), from a mask 0.92 -> 0.98, fp32 0.96 -> 1.03
-// (tests/gpu_dequant_tune.py, profiles/r02_dequant_ste_tune.json; outputs bit-identical for every grid).
+// (profiles/r02_dequant_ste_tune.json; outputs bit-identical for every grid).
 constexpr int kCtasPerSmDefault = 0;
 
 struct BwdParams {
@@ -218,15 +217,7 @@ int bwd_entry(const void* g, const void* x, const uint8_t* mask_in, void* gx, ui
     p.nvec = n / per;
     const int64_t tile = (int64_t)kThreads * kUnroll;
     int64_t grid = (p.nvec + tile - 1) / tile;
-    // grid cap in CTAs per SM (0 = one CTA per tile); QAT_B200_STE_TUNE=1 re-reads QAT_B200_STE_CTAS per call
-    // (tests/gpu_dequant_tune.py)
-    int ctas = kCtasPerSmDefault;
-    static const bool tune = [] { const char* e = getenv("QAT_B200_STE_TUNE"); return e != nullptr && e[0] == '1'; }();
-    if (tune) {
-      if (const char* e = getenv("QAT_B200_STE_CTAS")) ctas = atoi(e);
-      QAT_CHECK_ARG(ctas >= 0 && ctas <= 64, "QAT_B200_STE_CTAS must be in [0, 64]");
-    }
-    const int64_t cap = ctas > 0 ? (int64_t)sms * ctas : (int64_t)0x7fffffff;
+    const int64_t cap = kCtasPerSmDefault > 0 ? (int64_t)sms * kCtasPerSmDefault : (int64_t)0x7fffffff;
     if (grid > cap) grid = cap;
     if (grid < 1) grid = 1;
     if (dtype == QAT_F32)

@@ -477,52 +477,37 @@ class _QuantLinearFn(torch.autograd.Function):
         # MN-major A) with the STE pass-mask applied to the fp32 accumulator in the epilogue.
         # fp32 modules keep the library GEMM + mask kernel.
         own = dtype == torch.bfloat16 and N % 8 == 0 and K % 8 == 0 and g2.data_ptr() % 16 == 0
-        # The operands are rebuilt from the codes by one streaming pass each (qat_dequant_codes, 25 us for
-        # [11008, 4096]).  QAT_B200_BWD_DEQUANT_PASS=0 selects the variant that rebuilds them INSIDE the GEMM
-        # (converter warps, no dequantized tensor in HBM): bit-identical, but measured 2.1-2.5x slower at
-        # T = 2048 (336 vs 133 + 25 us for dgrad [2048 x 11008] x [11008 x 4096]) — every weight tile is converted
-        # T / 256 times instead of once and the converters, not the tensor pipe, pace the k-loop.
-        from_codes = own and K % 16 == 0 and os.environ.get("QAT_B200_BWD_DEQUANT_PASS", "1") == "0"
+        # The operands are rebuilt from the codes by one streaming pass each (qat_dequant_codes): DESIGN.md §4.
         gx = gw = None
         with _on(dev):
             stream = _stream_ptr(dev)
             if ctx.needs_input_grad[0]:
-                if from_codes:
+                wq = torch.empty((N, K), dtype=dtype, device=dev)       # == the reference's fake-quant W
+                check(L.qat_dequant_codes(wb, wb + we, wq.data_ptr(), N, K, dt, stream), "qat_dequant_codes")
+                if own:
                     gx = torch.empty((T, K), dtype=dtype, device=dev)
-                    check(L.qat_gemm_bf16_codes(g2.data_ptr(), wb, wb + we, gx.data_ptr(), xb + xm, T, K, N, 0, dt, 0,
-                                                stream), "qat_gemm_bf16_codes (dgrad)")
+                    check(L.qat_gemm_bf16(g2.data_ptr(), wq.data_ptr(), gx.data_ptr(), xb + xm, T, K, N, 0, 1,
+                                          dt, 0, stream), "qat_gemm_bf16 (dgrad)")
                 else:
-                    wq = torch.empty((N, K), dtype=dtype, device=dev)       # == the reference's fake-quant W
-                    check(L.qat_dequant_codes(wb, wb + we, wq.data_ptr(), N, K, dt, stream), "qat_dequant_codes")
-                    if own:
-                        gx = torch.empty((T, K), dtype=dtype, device=dev)
-                        check(L.qat_gemm_bf16(g2.data_ptr(), wq.data_ptr(), gx.data_ptr(), xb + xm, T, K, N, 0, 1,
-                                              dt, 0, stream), "qat_gemm_bf16 (dgrad)")
-                    else:
-                        t = torch.mm(g2, wq)
-                        gx = torch.empty_like(t)
-                        check(L.qat_ste_bwd_from_mask(t.data_ptr(), xb + xm, gx.data_ptr(), T * K, dt, stream),
-                              "qat_ste_bwd_from_mask")
-                    del wq
+                    t = torch.mm(g2, wq)
+                    gx = torch.empty_like(t)
+                    check(L.qat_ste_bwd_from_mask(t.data_ptr(), xb + xm, gx.data_ptr(), T * K, dt, stream),
+                          "qat_ste_bwd_from_mask")
+                del wq
                 gx = gx.view(ctx.in_shape)
             if ctx.needs_input_grad[1]:
-                if from_codes:
+                xq = torch.empty((T, K), dtype=dtype, device=dev)       # == the reference's fake-quant x
+                check(L.qat_dequant_codes(xb, xb + xe, xq.data_ptr(), T, K, dt, stream), "qat_dequant_codes")
+                if own:
                     gw = torch.empty((N, K), dtype=dtype, device=dev)
-                    check(L.qat_gemm_bf16_codes(g2.data_ptr(), xb, xb + xe, gw.data_ptr(), wb + wm, N, K, T, 1, dt, 0,
-                                                stream), "qat_gemm_bf16_codes (wgrad)")
+                    check(L.qat_gemm_bf16(g2.data_ptr(), xq.data_ptr(), gw.data_ptr(), wb + wm, N, K, T, 1, 1,
+                                          dt, 0, stream), "qat_gemm_bf16 (wgrad)")
                 else:
-                    xq = torch.empty((T, K), dtype=dtype, device=dev)       # == the reference's fake-quant x
-                    check(L.qat_dequant_codes(xb, xb + xe, xq.data_ptr(), T, K, dt, stream), "qat_dequant_codes")
-                    if own:
-                        gw = torch.empty((N, K), dtype=dtype, device=dev)
-                        check(L.qat_gemm_bf16(g2.data_ptr(), xq.data_ptr(), gw.data_ptr(), wb + wm, N, K, T, 1, 1,
-                                              dt, 0, stream), "qat_gemm_bf16 (wgrad)")
-                    else:
-                        t = torch.mm(g2.t(), xq)
-                        gw = torch.empty_like(t)
-                        check(L.qat_ste_bwd_from_mask(t.data_ptr(), wb + wm, gw.data_ptr(), N * K, dt, stream),
-                              "qat_ste_bwd_from_mask")
-                    del xq
+                    t = torch.mm(g2.t(), xq)
+                    gw = torch.empty_like(t)
+                    check(L.qat_ste_bwd_from_mask(t.data_ptr(), wb + wm, gw.data_ptr(), N * K, dt, stream),
+                          "qat_ste_bwd_from_mask")
+                del xq
         # mode 1 keeps a module's codes only from its forward to its backward (for the checkpoint
         # recompute in between): 1.125 B per weight element must not sit in HBM through the
         # optimizer step

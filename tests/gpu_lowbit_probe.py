@@ -18,7 +18,6 @@ from llm_qat_b200.utils_quant import _LowBitWeight  # noqa: E402
 from oracle import quant_oracle as qo  # noqa: E402
 
 PEAK = 6459.0
-THREADS = [0] + [int(t) for t in os.environ.get("LOWBIT_PROBE_THREADS", "").split(",") if t]
 try:
     PEAK = float(json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))["hbm_gbs"])
 except Exception:  # noqa: BLE001
@@ -62,25 +61,19 @@ def timing(steps=30):
                 def once(i):
                     _lib.check(L.qat_lowbit_weight_fwd(ws[i].data_ptr(), outs[i].data_ptr(), rows, cols, dt, bits, 0,
                                                        wsp.data_ptr(), wsp.numel(), st))
-                for thr in THREADS:
-                    if thr:
-                        os.environ["QAT_B200_LOWBIT_THREADS"] = str(thr)
-                    else:
-                        os.environ.pop("QAT_B200_LOWBIT_THREADS", None)
-                    for i in range(nbuf):
-                        once(i)
-                    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                    e0.record()
-                    for k in range(steps):
-                        once(k % nbuf)
-                    e1.record()
-                    e1.synchronize()
-                    us = e0.elapsed_time(e1) / steps * 1e3
-                    gbs = n * esz * 2 / us / 1e3
-                    key = f"{dt_name}[{rows},{cols}] W{bits}" + (f" threads={thr}" if thr else "")
-                    out[key] = {"us": round(us, 2), "GBps": round(gbs, 1), "frac": round(gbs / PEAK, 3)}
-                    print(f"{key}: {us:.1f} us  {gbs:.0f} GB/s  {gbs / PEAK:.3f} of peak", flush=True)
-                os.environ.pop("QAT_B200_LOWBIT_THREADS", None)
+                for i in range(nbuf):
+                    once(i)
+                e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                e0.record()
+                for k in range(steps):
+                    once(k % nbuf)
+                e1.record()
+                e1.synchronize()
+                us = e0.elapsed_time(e1) / steps * 1e3
+                gbs = n * esz * 2 / us / 1e3
+                key = f"{dt_name}[{rows},{cols}] W{bits}"
+                out[key] = {"us": round(us, 2), "GBps": round(gbs, 1), "frac": round(gbs / PEAK, 3)}
+                print(f"{key}: {us:.1f} us  {gbs:.0f} GB/s  {gbs / PEAK:.3f} of peak", flush=True)
             del ws, outs
     print(json.dumps({"lowbit_exact_kernel": out, "hbm_peak_GBps": PEAK}))
 

@@ -65,10 +65,6 @@ we = torch.rand(I, device=dev) * 100 + 50
 xc = torch.randint(-127, 128, (T, C), dtype=torch.int8, device=dev)
 xe = torch.rand(T, device=dev) * 100 + 50
 wq2, xq2 = torch.empty(I, C, device=dev).bfloat16(), torch.empty(T, C, device=dev).bfloat16()
-timed("dgrad_from_codes", lambda: _lib.check(L.qat_gemm_bf16_codes(
-    g.data_ptr(), wc.data_ptr(), we.data_ptr(), gx.data_ptr(), mx.data_ptr(), T, C, I, 0, 1, 0, st)), flops=2.0 * T * C * I)
-timed("wgrad_from_codes", lambda: _lib.check(L.qat_gemm_bf16_codes(
-    g.data_ptr(), xc.data_ptr(), xe.data_ptr(), gw.data_ptr(), mw.data_ptr(), I, C, T, 1, 1, 0, st)), flops=2.0 * T * C * I)
 timed("dequant_W[11008x4096]", lambda: _lib.check(L.qat_dequant_codes(wc.data_ptr(), we.data_ptr(), wq2.data_ptr(), I, C, 1, st)),
       nbytes=I * C * 3)
 timed("dequant_x[2048x4096]", lambda: _lib.check(L.qat_dequant_codes(xc.data_ptr(), xe.data_ptr(), xq2.data_ptr(), T, C, 1, st)),

@@ -1,7 +1,7 @@
 """GPU probe for qat_gemm_bf16 (csrc/gemm_bf16.cu): every operand majorness x CTA-group plan against
 an fp32 torch matmul, then timing against torch.mm (cuBLAS) at the QuantizeLinear backward shapes.
-Run on the GPU box:  python tests/gpu_umma_probe.py [--sweep-strides]
-Prints one JSON line per case; exits non-zero if a canonical-stride case is wrong."""
+Run on the GPU box:  python tests/gpu_umma_probe.py
+Prints one JSON line per case; exits non-zero if a case is wrong."""
 from __future__ import annotations
 
 import json
@@ -72,18 +72,6 @@ def main():
             ok &= good
             print(json.dumps({"masked": True, "shape": [M, N, K], "out": str(od), "rel_err": err, "ok": good}),
                   flush=True)
-    if "--sweep-strides" in sys.argv or not ok:
-        # which (LBO, SBO) does the hardware want for an MN-major operand?
-        for lbo, sbo in [(8192, 1024), (1024, 8192), (128, 1024), (1024, 128), (8192, 128), (16, 1024)]:
-            L.qat_gemm_bf16_debug_strides(lbo, sbo)
-            res = {}
-            for a_mn, b_mn in [(0, 1), (1, 0)]:
-                try:
-                    res[f"a{a_mn}b{b_mn}"] = case(256, 256, 128, a_mn, b_mn, 1)
-                except Exception as e:  # noqa: BLE001
-                    res[f"a{a_mn}b{b_mn}"] = repr(e)[:100]
-            print(json.dumps({"lbo": lbo, "sbo": sbo, **res}), flush=True)
-        L.qat_gemm_bf16_debug_strides(0, 0)
 
     # timing at the LLaMA-7B backward shapes (T = 2048 and 8192)
     def bench(fn, n=20):

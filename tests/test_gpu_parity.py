@@ -746,7 +746,6 @@ def test_quantize_linear_backward_runs_on_own_kernels(monkeypatch):
     from oracle import ref_module
 
     monkeypatch.setenv("QAT_B200_FUSED_LINEAR", "1")
-    monkeypatch.delenv("QAT_B200_BWD_DEQUANT_PASS", raising=False)
     gen = torch.Generator().manual_seed(9)
     T, K, N = 512, 1024, 1536
     x0 = (torch.randn(T, K, generator=gen) * 1.2).bfloat16().cuda()
@@ -1067,63 +1066,3 @@ def test_qkv_prep_position_ids_outside_the_tables_stay_in_bounds():
         qkv_prep(q0, k0[:, :32], v0, cos_t, sin_t, good, nh, 4)
     with pytest.raises(RuntimeError):
         qkv_prep(q0, k0, v0, cos_t.double(), sin_t, good, nh, 4)
-
-
-@pytest.mark.parametrize("a_mn", [0, 1])
-@pytest.mark.parametrize("cg", [1, 2])
-@pytest.mark.parametrize("shape", [(256, 256, 128), (304, 528, 200), (2048, 1024, 1088)])
-@pytest.mark.parametrize("amp", [False, True])
-def test_gemm_from_codes_is_bit_identical_to_dequant_then_gemm(a_mn, cg, shape, amp):
-    """qat_gemm_bf16_codes rebuilds B = fl_bf16(codes / e[row]) inside the kernel: its output must equal, bit
-    for bit, qat_dequant_codes followed by qat_gemm_bf16 on that tensor (same operands, same MMA order)."""
-    from llm_qat_b200 import _lib
-    from llm_qat_b200._lib import CODES_I8
-    from llm_qat_b200.utils_quant import dequant_codes, fake_quant_forward
-
-    M, N, K = shape
-    gen = torch.Generator().manual_seed(M + N)
-    A = torch.randn(M, K, generator=gen).bfloat16().cuda()
-    a = A.t().contiguous() if a_mn else A
-    src = (torch.randn(K, N, generator=gen) * 0.7).bfloat16().cuda()     # rows = contraction index
-    _, codes, _, e, mask_src = fake_quant_forward(src, 4, False, True, want_y=False, codes_kind=CODES_I8, want_scales=True,
-                                                  mask_clip=(-2.0, 2.0), amp=amp)
-    bits = torch.rand(M * N, generator=gen) < 0.8
-    mask = _pack_bits(bits).cuda()
-    st = torch.cuda.current_stream().cuda_stream
-    L = _lib.lib()
-    out1 = torch.empty(M, N, dtype=torch.bfloat16, device="cuda")
-    _lib.check(L.qat_gemm_bf16_codes(a.data_ptr(), codes.data_ptr(), e.data_ptr(), out1.data_ptr(), mask.data_ptr(), M, N, K,
-                                     a_mn, 1, cg, st), "qat_gemm_bf16_codes")
-    bq = dequant_codes(codes, e, torch.bfloat16)
-    out2 = torch.empty(M, N, dtype=torch.bfloat16, device="cuda")
-    _lib.check(L.qat_gemm_bf16(a.data_ptr(), bq.data_ptr(), out2.data_ptr(), mask.data_ptr(), M, N, K, a_mn, 1, 1, cg, st),
-               "qat_gemm_bf16")
-    assert torch.equal(out1, out2), (shape, a_mn, cg, float((out1.float() - out2.float()).abs().max()))
-    ref = (A.float() @ bq.float()) * bits.view(M, N).cuda()
-    assert ((out1.float() - ref).norm() / ref.norm()).item() <= 4e-3
-
-
-def test_quantize_linear_backward_in_gemm_dequant_variant_is_bit_identical(monkeypatch):
-    """QAT_B200_BWD_DEQUANT_PASS=0: operands rebuilt inside the contraction (no dequantized tensor in HBM) — the
-    gradients equal the default path's bit for bit, in two launches instead of four."""
-    from llm_qat_b200 import QuantizeLinear, _lib
-
-    gen = torch.Generator().manual_seed(13)
-    T, K, N = 384, 512, 768
-    x0 = (torch.randn(T, K, generator=gen) * 1.2).bfloat16().cuda()
-    w0 = (torch.randn(N, K, generator=gen) * 0.02).bfloat16().cuda()
-    g0 = torch.randn(T, N, generator=gen).bfloat16().cuda()
-    res = []
-    for mode in ("1", "0"):
-        monkeypatch.setenv("QAT_B200_BWD_DEQUANT_PASS", mode)
-        lin = QuantizeLinear(K, N, w_bits=4, a_bits=8).bfloat16().cuda()
-        with torch.no_grad():
-            lin.weight.copy_(w0)
-        x = x0.clone().requires_grad_(True)
-        with torch.autocast("cuda", dtype=torch.bfloat16):
-            out = lin(x)
-        n0 = _lib.launch_count()
-        out.backward(g0)
-        res.append((x.grad, lin.weight.grad, _lib.launch_count() - n0))
-    assert res[0][2] == 4 and res[1][2] == 2, (res[0][2], res[1][2])
-    assert torch.equal(res[0][0], res[1][0]) and torch.equal(res[0][1], res[1][1])
