@@ -163,9 +163,10 @@ int qat_qlinear_i8_fwd(const int8_t* qx, const int8_t* qw, const float* ex, cons
  * Also settable once through the environment, QAT_B200_PDL=0. */
 int qat_set_pdl(int enabled);
 
-/* Tuning knob of the contraction: CTAs per tcgen05.mma.  2 = CTA pairs on 256x256
- * tiles (cta_group::2), 1 = single CTAs on 128x256 tiles, 0 = choose per problem
- * (the default; also settable once through the environment, QAT_B200_GEMM_CG). */
+/* Tile plan of the tcgen05 GEMMs — qat_qlinear_i8_fwd, and qat_gemm_bf16 called with
+ * cta_group == 0: CTAs per tcgen05.mma.  2 = CTA pairs on 256x256 tiles (cta_group::2),
+ * 1 = single CTAs on 128x256 tiles, 0 = choose per problem (the default; also settable
+ * once through the environment, QAT_B200_GEMM_CG). */
 int qat_set_gemm_cta_group(int cta_group);
 
 /*
@@ -214,7 +215,7 @@ int qat_dequant_codes(const int8_t* codes, const float* row_e, void* out, int64_
  * mask (optional): packed pass-mask over the flattened [M, N] output, bit i%8 of byte i/8 (what
  * qat_sym_fwd emits); masked-out elements are written as 0.  out: bf16 or fp32 per out_dtype.
  * The contiguous dimension of each operand must be a multiple of 8 elements (TMA pitch).
- * cta_group: 0 = choose, 1 = 128x256 tiles, 2 = CTA pairs on 256x256 tiles.
+ * cta_group: 0 = choose (or what qat_set_gemm_cta_group set), 1 = 128x256 tiles, 2 = CTA pairs on 256x256 tiles.
  * tcgen05.mma kind::f16, TMEM accumulators, TMA-fed (MN-major shared-memory descriptors).
  */
 int qat_gemm_bf16(const void* a, const void* b, void* out, const uint8_t* mask, int64_t M, int64_t N,

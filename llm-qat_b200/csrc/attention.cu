@@ -897,18 +897,6 @@ int make_map_bshd(CUtensorMap* map, const void* ptr, int B, int S, int H, int bo
   return QAT_OK;
 }
 
-template <typename Kern>
-int set_smem(Kern kern, uint32_t bytes, bool* flags) {
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess) dev = 0;
-  if (dev < 0 || dev >= 64 || !flags[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(attention kernel)");
-    if (dev >= 0 && dev < 64) flags[dev] = true;
-  }
-  return QAT_OK;
-}
-
 int check_common(const void* q, const void* k, const void* v, int B, int S, int H, int Dh) {
   QAT_CHECK_ARG(Dh == D, "head_dim must be %d (got %d)", D, Dh);
   QAT_CHECK_ARG(B > 0 && S > 0 && H > 0, "bad shape B=%d S=%d H=%d", B, S, H);
@@ -936,8 +924,8 @@ extern "C" int qat_attn_fwd(const void* q, const void* k, const void* v, void* o
   if ((rc = make_map_bshd(&mq, q, B, S, H, BM)) != QAT_OK) return rc;
   if ((rc = make_map_bshd(&mk, k, B, S, H, BM)) != QAT_OK) return rc;
   if ((rc = make_map_bshd(&mv, v, B, S, H, BM)) != QAT_OK) return rc;
-  static bool flags[64] = {};
-  if ((rc = set_smem(attn_fwd_kernel, fwd::kSmem, flags)) != QAT_OK) return rc;
+  static bool opted_in[64] = {};
+  if ((rc = opt_in_smem(attn_fwd_kernel, fwd::kSmem, opted_in, "attention kernel")) != QAT_OK) return rc;
   AttnParams p{};
   p.trace = g_attn_trace;
   p.o = o;
@@ -991,8 +979,8 @@ extern "C" int qat_attn_bwd(const void* q, const void* k, const void* v, const v
     if ((rc = make_map_bshd(&mdo, d_o, B, S, H, BM)) != QAT_OK) return rc;
     if ((rc = make_map_bshd(&mk, k, B, S, H, bq::BN)) != QAT_OK) return rc;
     if ((rc = make_map_bshd(&mv, v, B, S, H, bq::BN)) != QAT_OK) return rc;
-    static bool flags[64] = {};
-    if ((rc = set_smem(attn_bwd_dq_kernel, bq::kSmem, flags)) != QAT_OK) return rc;
+    static bool opted_in[64] = {};
+    if ((rc = opt_in_smem(attn_bwd_dq_kernel, bq::kSmem, opted_in, "attention kernel")) != QAT_OK) return rc;
     const dim3 grid((unsigned)((S + BM - 1) / BM), (unsigned)H, (unsigned)B);
     cudaError_t e = launch_pdl(attn_bwd_dq_kernel, grid, dim3(bq::kThreads), bq::kSmem, st, mq, mk, mv, mdo, p);
     if (e != cudaSuccess) return cuda_fail(e, "attn_bwd_dq_kernel launch");
@@ -1004,8 +992,8 @@ extern "C" int qat_attn_bwd(const void* q, const void* k, const void* v, const v
     if ((rc = make_map_bshd(&mdo, d_o, B, S, H, bk::BN)) != QAT_OK) return rc;
     if ((rc = make_map_bshd(&mk, k, B, S, H, BM)) != QAT_OK) return rc;
     if ((rc = make_map_bshd(&mv, v, B, S, H, BM)) != QAT_OK) return rc;
-    static bool flags[64] = {};
-    if ((rc = set_smem(attn_bwd_dkv_kernel, bk::kSmem, flags)) != QAT_OK) return rc;
+    static bool opted_in[64] = {};
+    if ((rc = opt_in_smem(attn_bwd_dkv_kernel, bk::kSmem, opted_in, "attention kernel")) != QAT_OK) return rc;
     const dim3 grid((unsigned)((S + BM - 1) / BM), (unsigned)H, (unsigned)B);
     cudaError_t e = launch_pdl(attn_bwd_dkv_kernel, grid, dim3(bk::kThreads), bk::kSmem, st, mq, mk, mv, mdo, p);
     if (e != cudaSuccess) return cuda_fail(e, "attn_bwd_dkv_kernel launch");

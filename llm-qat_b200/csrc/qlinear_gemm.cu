@@ -7,74 +7,20 @@
 // emits in its codes-only mode.  The integer dot product is exact (s32
 // accumulators), so the result is at least as accurate as the reference's.
 //
-// sm_100a design (template parameter CG = CTAs per MMA, the PTX cta_group)
-//   * persistent grid, one CTA per SM, static round-robin over output tiles;
-//   * CG == 2 (default for large problems): the two CTAs of a cluster (one TPC)
-//     own one 256x256 tile.  Each CTA stages its own 128 rows of A and its own
-//     128-row half of B (32 KB per k-block instead of 48 KB) and holds 128 rows
-//     of the accumulator in its TMEM; the leader CTA issues
-//     tcgen05.mma.cta_group::2 (M256 x N256 x K32), which reads B from both
-//     CTAs' shared memory.  Per SM the operand read rate drops from 96 to
-//     64 B/clk — below the 128 B/clk shared-memory port — which is what lets the
-//     tensor pipe stay busy (the CG == 1 kernel measured 75 % tensor-active).
-//   * CG == 1: one CTA per 128x256 tile (small problems, odd SM counts).
-//   * warp 0   : TMA producer  (cp.async.bulk.tensor.2d, 128B swizzle; with
-//                               CG == 2 both CTAs' loads complete on the
-//                               leader's mbarrier)
-//   * warp 1   : MMA issuer    (one thread of the leader CTA, kind::i8, s32
-//                               accumulators in TMEM; tcgen05.commit multicasts
-//                               "stage free" / "accumulator full" to both CTAs)
-//   * warp 2   : TMEM allocator (512 columns = 2 accumulator stages)
-//   * warps 4-7: epilogue      (tcgen05.ld 32x32b.x32 -> I2F -> x row/col
-//                               scales -> bf16/fp32 -> 16-byte global stores),
-//                               overlapped with the next tile's MMAs.
-//   * smem: CG1 4 x (16 KB A + 32 KB B), CG2 6 x (16 KB A + 16 KB B), plus
-//     column-scale staging = ~195 KB.
+// The pipeline is tcgen05_gemm.cuh's (kind::i8, s32 accumulators in TMEM, both operands
+// K-major); what is specific to K4 is the dual-scale epilogue: the epilogue warps stage 1/ew for
+// the tile's 256 columns in shared memory while the MMAs run, then each 32-column chunk goes
+// I2F -> x 1/ex[row] -> x 1/ew[col] -> bf16/fp32.  The output type is a template parameter.
 // Tensor-bound: 2*T*N*K integer ops; see DESIGN.md "K4".
 #define QAT_PDL_FAMILY 4   // bit of QAT_B200_PDL_MASK (common.cuh)
 #include <cstdlib>
 
-#include "umma.cuh"
+#include "tcgen05_gemm.cuh"
 
 namespace qat {
 namespace {
 
-constexpr int BLOCK_M = 128;  // accumulator rows per CTA (TMEM lanes)
-constexpr int BLOCK_N = 256;  // accumulator columns per tile
 constexpr int BLOCK_K = 128;  // bytes == int8 elements: one 128B swizzle row
-constexpr int UMMA_K = 32;    // elements per tcgen05.mma.kind::i8
-constexpr int kAccStages = 2;
-constexpr int kTmemCols = kAccStages * BLOCK_N;  // 512
-constexpr int kThreads = 256;
-constexpr int kEpiWarp0 = 4;  // warps 4..7; (warp % 4) selects the TMEM lane quadrant
-constexpr int kEpiThreads = 128;
-constexpr int kEpiWarps = kEpiThreads / 32;
-
-// Per-CTA shared-memory plan.  CG CTAs cooperate on one (CG*128) x 256 tile.
-template <int CG>
-struct Cfg {
-  static constexpr int kStages = CG == 1 ? 4 : 6;
-  static constexpr int kTileM = BLOCK_M * CG;                    // output rows per tile
-  static constexpr int kBRows = BLOCK_N / CG;                    // B rows staged by each CTA
-  static constexpr uint32_t kABytes = BLOCK_M * BLOCK_K;         // 16 KB
-  static constexpr uint32_t kBBytes = kBRows * BLOCK_K;          // 32 KB | 16 KB
-  static constexpr uint32_t kStageBytes = kABytes + kBBytes;
-  // offsets from the 1024-byte aligned base (identical in both CTAs of a pair)
-  static __host__ __device__ constexpr uint32_t a(int s) { return (uint32_t)s * kStageBytes; }
-  static __host__ __device__ constexpr uint32_t b(int s) { return (uint32_t)s * kStageBytes + kABytes; }
-  static constexpr uint32_t colscale = kStages * kStageBytes;             // 2 x 256 floats
-  static constexpr uint32_t bars = colscale + kAccStages * BLOCK_N * 4;   // 8-byte aligned
-  static __host__ __device__ constexpr uint32_t full(int s) { return bars + 8u * s; }
-  static __host__ __device__ constexpr uint32_t empty(int s) { return bars + 8u * (kStages + s); }
-  static __host__ __device__ constexpr uint32_t tfull(int a) { return bars + 8u * (2 * kStages + a); }
-  static __host__ __device__ constexpr uint32_t tempty(int a) { return bars + 8u * (2 * kStages + kAccStages + a); }
-  static constexpr uint32_t tmem_ptr = bars + 8u * (2 * kStages + 2 * kAccStages);
-  static constexpr uint32_t total = tmem_ptr + 16;
-  static constexpr uint32_t kSmemBytes = total + 1024;  // slack for manual 1024B alignment
-};
-static_assert(Cfg<1>::kSmemBytes <= 232448 && Cfg<2>::kSmemBytes <= 232448, "over the 227 KB per-CTA limit");
-
-using namespace umma;  // mbarrier / TMA / tcgen05 wrappers, descriptors
 
 struct GemmParams {
   const float* ex;  // [T] dequant divisors of the activation rows
@@ -85,294 +31,79 @@ struct GemmParams {
 };
 
 template <int OUT_DT>
-__device__ __forceinline__ void store_chunk(const GemmParams& p, int64_t row, int64_t col0,
-                                            const uint32_t (&acc)[32], float row_scale,
-                                            const float* colscale /* smem, 32 entries */, bool vec_ok) {
-  float v[32];
+struct I8Op {
+  using Params = GemmParams;
+  static constexpr int kBlockK = BLOCK_K;
+  static constexpr int kUmmaK = 32;   // elements per tcgen05.mma.kind::i8
+  static constexpr bool kAMN = false, kBMN = false;
+  static constexpr uint32_t kEpiBytes = kAccStages * BLOCK_N * 4;   // 1/ew of each accumulator stage's columns
+  static constexpr bool kStopPastN = false;
+  static __host__ __device__ constexpr uint32_t idesc(int m) { return make_idesc_i8(m, BLOCK_N); }
+  template <int CG>
+  static __device__ __forceinline__ void mma(uint32_t d, uint64_t a, uint64_t b, uint32_t idesc, uint32_t acc) {
+    umma_i8<CG>(d, a, b, idesc, acc);
+  }
+  static __device__ __forceinline__ bool out_bf16(const Params&) { return OUT_DT == QAT_BF16; }
+
+  struct Tile {
+    const float* colscale;  // smem, 256 entries
+    float row_scale;
+  };
+  static __device__ __forceinline__ Tile tile_prologue(const Params& p, uint8_t* epi, int acc, int64_t row,
+                                                       int64_t col_base) {
+    const int et = threadIdx.x - kEpiWarp0 * 32;  // 0..127
+    float* colscale = reinterpret_cast<float*>(epi) + acc * BLOCK_N;
+    // stage 1/ew for this tile's 256 columns (2 per thread) while the MMAs run
 #pragma unroll
-  for (int j = 0; j < 32; ++j)
-    v[j] = __fmul_rn(__fmul_rn((float)(int32_t)acc[j], row_scale), colscale[j]);
-  if (OUT_DT == QAT_BF16) {
-    __nv_bfloat16* dst = reinterpret_cast<__nv_bfloat16*>(p.out) + row * p.N + col0;
-    if (vec_ok && col0 + 32 <= p.N) {
-#pragma unroll
-      for (int j = 0; j < 32; j += 8) {
-        uint4 o;
-        o.x = pack_bf16x2(v[j], v[j + 1]);
-        o.y = pack_bf16x2(v[j + 2], v[j + 3]);
-        o.z = pack_bf16x2(v[j + 4], v[j + 5]);
-        o.w = pack_bf16x2(v[j + 6], v[j + 7]);
-        *reinterpret_cast<uint4*>(dst + j) = o;
-      }
-    } else {
-#pragma unroll
-      for (int j = 0; j < 32; ++j)
-        if (col0 + j < p.N) dst[j] = __float2bfloat16_rn(v[j]);
+    for (int j = et; j < BLOCK_N; j += kEpiThreads) {
+      const int64_t c = col_base + j;
+      colscale[j] = (c < p.N) ? __frcp_rn(p.ew[c]) : 0.f;
     }
-  } else {
-    float* dst = reinterpret_cast<float*>(p.out) + row * p.N + col0;
-    if (vec_ok && col0 + 32 <= p.N) {
-#pragma unroll
-      for (int j = 0; j < 32; j += 4)
-        *reinterpret_cast<float4*>(dst + j) = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
-    } else {
+    const float row_scale = (row < p.T) ? __frcp_rn(p.ex[row]) : 0.f;
+    asm volatile("bar.sync 1, %0;" ::"n"(kEpiThreads) : "memory");  // colscale visible to the 4 warps
+    return {colscale, row_scale};
+  }
+  static __device__ __forceinline__ void store(const Params& p, const Tile& t, int64_t row, int64_t col0, int c,
+                                               const uint32_t (&acc)[32], bool vec_ok) {
+    if (row < p.T && col0 < p.N) {
+      float v[32];
 #pragma unroll
       for (int j = 0; j < 32; ++j)
-        if (col0 + j < p.N) dst[j] = v[j];
+        v[j] = __fmul_rn(__fmul_rn((float)(int32_t)acc[j], t.row_scale), t.colscale[c * 32 + j]);
+      store_row32(p.out, OUT_DT == QAT_BF16, row, col0, p.N, v, vec_ok);
     }
   }
-}
+};
 
 template <int OUT_DT, int CG>
 __global__ void __launch_bounds__(kThreads, 1)
 qlinear_i8_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
                   const GemmParams p) {
-  using C = Cfg<CG>;
-  extern __shared__ uint8_t smem_raw[];
-  // the dynamic window starts at the same shared::cta offset in every CTA of the
-  // kernel, so `base` — and with it every barrier / tile offset — is identical
-  // in both CTAs of a pair (the multicast commit and the peer-bit trick need it)
-  const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* base_ptr = smem_raw + (base - smem_u32(smem_raw));
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = (CG == 2) ? cluster_ctarank() : 0u;   // 0 = leader (issues the MMAs)
-  const int unit = (CG == 2) ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;   // CTA (pair) index
-  const int num_units = (CG == 2) ? (int)(gridDim.x >> 1) : (int)gridDim.x;
-  const int num_tiles = p.m_blocks * p.n_blocks;
-
-  if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_a) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_b) : "memory");
-  }
-  if (warp == 1 && lane == 0) {
-#pragma unroll
-    for (int s = 0; s < C::kStages; ++s) {
-      mbar_init(base + C::full(s), 1);    // the leader's producer: arrive.expect_tx (bytes of both CTAs)
-      mbar_init(base + C::empty(s), 1);   // one tcgen05.commit arrival (multicast to both CTAs when CG == 2)
-    }
-#pragma unroll
-    for (int a = 0; a < kAccStages; ++a) {
-      mbar_init(base + C::tfull(a), 1);
-      mbar_init(base + C::tempty(a), CG * kEpiWarps);   // one arrival per epilogue warp of every CTA
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 2) {
-    if (CG == 1) {
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(base + C::tmem_ptr),
-                   "n"(kTmemCols)
-                   : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    } else {
-      asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(base + C::tmem_ptr),
-                   "n"(kTmemCols)
-                   : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    }
-  }
-  tcgen05_fence_before();
-  if (CG == 2) cluster_sync_all(); else __syncthreads();   // peers touch our barriers: cluster-wide
-  tcgen05_fence_after();
-  const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(base_ptr + C::tmem_ptr);
-  // barrier init, TMEM allocation and descriptor prefetch above overlap the previous
-  // kernel's tail; its results (the codes K1 wrote) are read only from here on
-  pdl_wait();
-  pdl_launch_dependents();
-
-  if (warp == 0) {
-    // ===================== TMA producer (every CTA loads its own rows) =====================
-    if (lane == 0) {
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int tile = unit; tile < num_tiles; tile += num_units) {
-        const int m_blk = tile % p.m_blocks, n_blk = tile / p.m_blocks;
-        const int32_t a_row = m_blk * C::kTileM + (int)rank * BLOCK_M;
-        const int32_t b_row = n_blk * BLOCK_N + (int)rank * C::kBRows;
-        for (int kb = 0; kb < p.k_blocks; ++kb) {
-          mbar_wait(base + C::empty(stage), phase ^ 1u);   // own copy: the commit is multicast
-          const uint32_t full = base + C::full(stage);
-          if (CG == 1) {
-            mbar_expect_tx(full, C::kStageBytes);
-            tma_load_2d(base + C::a(stage), &map_a, full, kb * BLOCK_K, a_row);
-            tma_load_2d(base + C::b(stage), &map_b, full, kb * BLOCK_K, b_row);
-          } else {
-            if (rank == 0) mbar_expect_tx(full, 2 * C::kStageBytes);
-            tma_load_2d_pair(base + C::a(stage), &map_a, full, kb * BLOCK_K, a_row);
-            tma_load_2d_pair(base + C::b(stage), &map_b, full, kb * BLOCK_K, b_row);
-          }
-          if (++stage == C::kStages) {
-            stage = 0;
-            phase ^= 1u;
-          }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ===================== MMA issuer (single thread of the leader CTA) =====================
-    if (lane == 0 && rank == 0) {
-      constexpr uint32_t idesc = make_idesc_i8(C::kTileM, BLOCK_N);
-      int stage = 0, acc = 0;
-      uint32_t phase = 0, acc_phase = 0;
-      for (int tile = unit; tile < num_tiles; tile += num_units) {
-        mbar_wait(base + C::tempty(acc), acc_phase ^ 1u);  // every epilogue warp drained this stage
-        tcgen05_fence_after();
-        const uint32_t tmem_d = tmem_base + (uint32_t)(acc * BLOCK_N);
-        for (int kb = 0; kb < p.k_blocks; ++kb) {
-          mbar_wait(base + C::full(stage), phase);
-          tcgen05_fence_after();
-          const uint64_t adesc = make_smem_desc(base + C::a(stage));
-          const uint64_t bdesc = make_smem_desc(base + C::b(stage));
-#pragma unroll
-          for (int k = 0; k < BLOCK_K / UMMA_K; ++k) {
-            // advance 32 bytes inside the 128B swizzle atom: +2 in the (>>4) address field
-            umma_i8<CG>(tmem_d, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc,
-                        (kb > 0 || k > 0) ? 1u : 0u);
-          }
-          // frees the smem stage (in both CTAs) when the MMAs retire
-          if (CG == 1) umma_commit(base + C::empty(stage)); else umma_commit_pair(base + C::empty(stage));
-          if (++stage == C::kStages) {
-            stage = 0;
-            phase ^= 1u;
-          }
-        }
-        // accumulator complete -> epilogue (of both CTAs)
-        if (CG == 1) umma_commit(base + C::tfull(acc)); else umma_commit_pair(base + C::tfull(acc));
-        if (++acc == kAccStages) {
-          acc = 0;
-          acc_phase ^= 1u;
-        }
-      }
-    }
-  } else if (warp >= kEpiWarp0) {
-    // ===================== epilogue (4 warps, 128 threads, own 128 accumulator rows) =====================
-    const int quad = warp & 3;              // TMEM lane quadrant this warp may read
-    const int et = threadIdx.x - kEpiWarp0 * 32;  // 0..127
-    const bool vec_ok = (OUT_DT == QAT_BF16) ? (p.N % 8 == 0) : (p.N % 4 == 0);
-    int acc = 0;
-    uint32_t acc_phase = 0;
-    for (int tile = unit; tile < num_tiles; tile += num_units) {
-      const int m_blk = tile % p.m_blocks, n_blk = tile / p.m_blocks;
-      const int64_t row = (int64_t)m_blk * C::kTileM + (int64_t)rank * BLOCK_M + quad * 32 + lane;
-      const int64_t col_base = (int64_t)n_blk * BLOCK_N;
-      float* colscale = reinterpret_cast<float*>(base_ptr + C::colscale) + acc * BLOCK_N;
-      // stage 1/ew for this tile's 256 columns (2 per thread) while the MMAs run
-#pragma unroll
-      for (int j = et; j < BLOCK_N; j += kEpiThreads) {
-        const int64_t c = col_base + j;
-        colscale[j] = (c < p.N) ? __frcp_rn(p.ew[c]) : 0.f;
-      }
-      const float row_scale = (row < p.T) ? __frcp_rn(p.ex[row]) : 0.f;
-      asm volatile("bar.sync 1, %0;" ::"n"(kEpiThreads) : "memory");  // colscale visible to the 4 warps
-      mbar_wait(base + C::tfull(acc), acc_phase);
-      tcgen05_fence_after();
-      const uint32_t taddr = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(acc * BLOCK_N);
-#pragma unroll 1
-      for (int c = 0; c < BLOCK_N / 32; ++c) {
-        uint32_t r[32];
-        tmem_ld_32x32b_x32(taddr + (uint32_t)(c * 32), r);
-        tmem_ld_wait();
-        if (row < p.T && col_base + c * 32 < p.N)
-          store_chunk<OUT_DT>(p, row, col_base + c * 32, r, row_scale, colscale + c * 32, vec_ok);
-      }
-      tcgen05_fence_before();
-      __syncwarp();
-      if (lane == 0) {
-        if (CG == 1) mbar_arrive(base + C::tempty(acc)); else mbar_arrive_remote(base + C::tempty(acc), 0u);
-      }
-      if (++acc == kAccStages) {
-        acc = 0;
-        acc_phase ^= 1u;
-      }
-    }
-  }
-
-  tcgen05_fence_before();
-  if (CG == 2) cluster_sync_all(); else __syncthreads();   // nobody leaves while its peer may still use it
-  if (warp == 2) {
-    tcgen05_fence_after();
-    if (CG == 1)
-      asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(kTmemCols)
-                   : "memory");
-    else
-      asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(kTmemCols)
-                   : "memory");
-  }
-}
-
-// ---- host: tensor maps --------------------------------------------------------
-// [rows, K] int8 row-major -> 2-D map, box = {128 bytes of K, box_rows}, 128B swizzle
-int make_map(CUtensorMap* map, const void* ptr, int64_t rows, int64_t K, int box_rows) {
-  EncodeFn enc = get_encode();
-  if (enc == nullptr) {
-    set_error("cuTensorMapEncodeTiled is not available from the CUDA driver");
-    return QAT_ERR_UNSUPPORTED;
-  }
-  cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)K};  // bytes between rows (int8)
-  cuuint32_t box[2] = {(cuuint32_t)BLOCK_K, (cuuint32_t)box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void*>(ptr), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled failed (CUresult %d) for [%lld, %lld] int8", (int)r, (long long)rows,
-              (long long)K);
-    return QAT_ERR_BAD_ARG;
-  }
-  return QAT_OK;
+  gemm_body<I8Op<OUT_DT>, CG>(map_a, map_b, p);
 }
 
 template <int OUT_DT, int CG>
 int launch(const CUtensorMap& ma, const CUtensorMap& mb, const GemmParams& p, cudaStream_t st) {
-  using C = Cfg<CG>;
-  // the opt-in to > 48 KB of dynamic shared memory is per function AND per device
-  static bool attr_set[64] = {};  // per instantiation; benign race (idempotent)
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess) dev = 0;
-  if (dev < 0 || dev >= 64 || !attr_set[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(qlinear_i8_kernel<OUT_DT, CG>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)C::kSmemBytes);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(qlinear_i8_kernel)");
-    if (dev >= 0 && dev < 64) attr_set[dev] = true;
-  }
-  const int tiles = p.m_blocks * p.n_blocks;
-  int units = num_sms() / CG;   // one CTA (pair) per SM (TPC)
-  if (units > tiles) units = tiles;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)(units * CG));
-  cfg.blockDim = dim3(kThreads);
-  cfg.dynamicSmemBytes = C::kSmemBytes;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CG;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = pdl_enabled(QAT_PDL_FAMILY) ? 1 : 0;
-  cfg.attrs = attr;
-  cfg.numAttrs = 2;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, qlinear_i8_kernel<OUT_DT, CG>, ma, mb, p);
-  if (e != cudaSuccess) return cuda_fail(e, "qlinear_i8_kernel launch");
-  QAT_CHECK_LAUNCH("qlinear_i8_kernel");
-  return QAT_OK;
+  return launch_gemm<I8Op<OUT_DT>, CG>(qlinear_i8_kernel<OUT_DT, CG>, "qlinear_i8_kernel", ma, mb, p, st,
+                                       QAT_PDL_FAMILY);
 }
 
-// CTAs per MMA for a problem: pairs pay off once there are enough 256-row tiles
-// to fill the machine; QAT_B200_GEMM_CG=1|2 forces a choice (tests, profiling).
-int g_forced_cg = -1;  // -1: not yet read from the environment; 0: automatic
-int pick_cta_group(int64_t T, int64_t N) {
+// 0: automatic; -1: not yet read from the environment
+int g_forced_cg = -1;
+
+}  // namespace
+
+int pick_cta_group(int64_t M, int64_t N) {
   if (g_forced_cg < 0) {
     const char* v = getenv("QAT_B200_GEMM_CG");
     g_forced_cg = (v && (v[0] == '1' || v[0] == '2')) ? v[0] - '0' : 0;
   }
   if (g_forced_cg) return g_forced_cg;
   if (num_sms() % 2) return 1;
-  const int64_t pair_tiles = ((T + 255) / 256) * ((N + BLOCK_N - 1) / BLOCK_N);
+  const int64_t pair_tiles = ((M + 255) / 256) * ((N + BLOCK_N - 1) / BLOCK_N);
   return pair_tiles >= num_sms() / 2 ? 2 : 1;
 }
 
-}  // namespace
 }  // namespace qat
 
 extern "C" int qat_set_gemm_cta_group(int cta_group) {
@@ -396,9 +127,9 @@ extern "C" int qat_qlinear_i8_fwd(const int8_t* qx, const int8_t* qw, const floa
   QAT_CHECK_ARG(T < (1ll << 31) && N < (1ll << 31) && K < (1ll << 31), "dimension too large");
   const int cg = pick_cta_group(T, N);
   CUtensorMap ma, mb;
-  int rc = make_map(&ma, qx, T, K, BLOCK_M);
+  int rc = make_map_2d(&ma, 1, qx, T, K, K, BLOCK_M);
   if (rc != QAT_OK) return rc;
-  rc = make_map(&mb, qw, N, K, BLOCK_N / cg);
+  rc = make_map_2d(&mb, 1, qw, N, K, K, BLOCK_N / cg);
   if (rc != QAT_OK) return rc;
   GemmParams p{};
   p.ex = ex;

@@ -1,7 +1,7 @@
 // umma.cuh — PTX wrappers shared by the tcgen05 kernels of libqat_b200 (sm_100a):
 // mbarriers, TMA (cp.async.bulk.tensor), tcgen05.mma / commit / ld / st, TMEM
 // allocation, shared-memory matrix descriptors and instruction descriptors.
-// Used by qlinear_gemm.cu (K4, kind::i8), gemm_bf16.cu (dgrad / wgrad, kind::f16)
+// Used by tcgen05_gemm.cuh (the GEMM pipeline of qlinear_gemm.cu and gemm_bf16.cu)
 // and attention.cu (QK^T / PV and their backward, kind::f16).
 #pragma once
 #include <cuda.h>
@@ -277,26 +277,45 @@ inline EncodeFn get_encode() {
   return fn;
 }
 
-// Row-major bf16 matrix [rows, cols] with a row pitch of `pitch_elems` -> 2-D map with a
-// {64 elements (128 B), box_rows} box, 128B swizzle.  OOB reads fill zeros.
-inline int make_map_bf16_2d(CUtensorMap* map, const void* ptr, int64_t rows, int64_t cols, int64_t pitch_elems,
-                            int box_rows) {
+// Row-major matrix [rows, cols] of bf16 (elem_bytes = 2) or int8 (elem_bytes = 1) with a row pitch
+// of `pitch_elems` -> 2-D map with a {128 B, box_rows} box, 128B swizzle.  OOB reads fill zeros.
+inline int make_map_2d(CUtensorMap* map, int elem_bytes, const void* ptr, int64_t rows, int64_t cols,
+                       int64_t pitch_elems, int box_rows) {
   EncodeFn enc = get_encode();
   if (enc == nullptr) {
     set_error("cuTensorMapEncodeTiled is not available from the CUDA driver");
     return QAT_ERR_UNSUPPORTED;
   }
+  const bool bf16 = elem_bytes == 2;
   cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)pitch_elems * 2};
-  cuuint32_t box[2] = {64u, (cuuint32_t)box_rows};
+  cuuint64_t strides[1] = {(cuuint64_t)pitch_elems * elem_bytes};
+  cuuint32_t box[2] = {128u / elem_bytes, (cuuint32_t)box_rows};
   cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  CUresult r = enc(map, bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_UINT8, 2,
+                   const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled failed (CUresult %d) for bf16 [%lld, %lld] pitch %lld box_rows %d", (int)r,
-              (long long)rows, (long long)cols, (long long)pitch_elems, box_rows);
+    set_error("cuTensorMapEncodeTiled failed (CUresult %d) for %s [%lld, %lld] pitch %lld box_rows %d", (int)r,
+              bf16 ? "bf16" : "int8", (long long)rows, (long long)cols, (long long)pitch_elems, box_rows);
     return QAT_ERR_BAD_ARG;
+  }
+  return QAT_OK;
+}
+
+// The opt-in to more than 48 KB of dynamic shared memory is per function AND per device.  `done`
+// is the caller's per-kernel record of the devices already opted in (a benign race: idempotent).
+template <typename Kern>
+int opt_in_smem(Kern kern, uint32_t bytes, bool (&done)[64], const char* name) {
+  int dev = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess) dev = 0;
+  if (dev < 0 || dev >= 64 || !done[dev]) {
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    if (e != cudaSuccess) {
+      char what[96];
+      snprintf(what, sizeof(what), "cudaFuncSetAttribute(%s)", name);
+      return cuda_fail(e, what);
+    }
+    if (dev >= 0 && dev < 64) done[dev] = true;
   }
   return QAT_OK;
 }
